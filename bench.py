@@ -10,7 +10,7 @@ dist.gather + unpack as the A/B.  A "ray" is one reference castRay call (primary
 secondary; reference src/scene.cpp:65,91,127,134).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl reference]
-                  [--assemble peer|nccl] [--configs all|none]
+                  [--assemble peer|nccl] [--configs all|none] [--dump-outputs DIR]
 
 N > 1 is launched by the driver with torch.distributed.run (one rank per GPU, NCCL).
 `--impl reference` times the reference's own CPU implementation of the path
@@ -280,6 +280,27 @@ def parity_check(pkg, ren, wl_name):
             "ray_count_equal": bool(count_ok), "max_abs_diff_fp64": err, "ok": bool(ids_ok and count_ok and err <= 1e-9)}
 
 
+DUMP_PIXELS = 1 << 21      # --dump-outputs: frames up to this many pixels whole, larger ones as a sample of this size
+
+
+def dump_outputs(out_dir, frame, height, width, rays_cls):
+    """What the timed path returned in its last step, for comparing two builds output for output: the RGB8 frame as
+    float32 (frame_rgb8.npy, H x W x 3), or for a frame of more than DUMP_PIXELS pixels the pixels at fixed positions
+    (seed 0, sorted; frame_rgb8_sample.npy, n x 3, and their row-major indices in frame_sample_index.npy), and the
+    primary / shadow / secondary ray counts (rays_per_class.npy).  At most 42 MB in all."""
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    if frame is not None:
+        img = frame.cpu().numpy().reshape(height * width, 3)
+        if height * width <= DUMP_PIXELS:
+            np.save(out / "frame_rgb8.npy", img.reshape(height, width, 3).astype(np.float32))
+        else:
+            idx = np.unique(np.random.default_rng(0).integers(0, height * width, DUMP_PIXELS))
+            np.save(out / "frame_rgb8_sample.npy", img[idx].astype(np.float32))
+            np.save(out / "frame_sample_index.npy", idx.astype(np.float64))
+    np.save(out / "rays_per_class.npy", np.array(rays_cls, np.float64))
+
+
 def load_traffic(wl_name):
     tf = ROOT / "profiles" / "traffic.json"
     try:
@@ -436,6 +457,8 @@ def run_workload(args, pkg, torch, dist, wl_name, headline):
     rays_frame = sum(rays_cls)
     launches_total = int(rays[3].item())
     value = rays_frame * steps / (ms_total * 1e-3) / 1e6
+    if args.dump_outputs and headline and rank == 0:
+        dump_outputs(args.dump_outputs, frame, height, width, rays_cls)
 
     # ---------------- the assembled frame against a single-rank render of the same frame (rank 0, after the timed region)
     frame_check = None
@@ -695,8 +718,10 @@ def run_workload(args, pkg, torch, dist, wl_name, headline):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
-    ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--steps", type=int, default=10,
+                    help="timed steps of the headline workload (the other configs of --configs all time min(K, 5))")
+    ap.add_argument("--warmup", type=int, default=3,
+                    help="untimed steps before them (the other configs warm up with 3)")
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="synthetic", choices=sorted(WORKLOADS))
     ap.add_argument("--assemble", default="peer", choices=["peer", "nccl"],
@@ -707,7 +732,11 @@ def main():
                     help="single process: render with rt_params.n_gpus = N (the library drives N GPUs itself); not the driver's launch mode")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the headline workload's output of its last timed step to DIR/*.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

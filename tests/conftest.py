@@ -169,8 +169,15 @@ def oracle(pkg):
 @pytest.fixture(scope="session")
 def reference():
     if not Reference.available():
-        pytest.skip("oracle/_ref/libref.so not built (needs /root/reference at build time)")
+        pytest.skip("oracle/_ref/libref.so not built (needs the reference sources at build time, oracle/Makefile REF=)")
     return Reference()
+
+
+@pytest.fixture(scope="session")
+def live_reference():
+    """The live reference where oracle/_ref is built, else None: for tests whose checks stand without it and that
+    also compare with it when they can."""
+    return Reference() if Reference.available() else None
 
 
 @pytest.fixture(scope="session")

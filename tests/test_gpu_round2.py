@@ -422,7 +422,7 @@ def test_pathb_reference_main_on_the_b200(tmp_path):
     from conftest import ORACLE_DIR, decode_png
     exe = ORACLE_DIR / "_ref" / "as2_pathb"
     if not exe.exists():
-        pytest.skip("oracle/_ref/as2_pathb not built (needs /root/reference at build time)")
+        pytest.skip("oracle/_ref/as2_pathb not built (needs the reference sources at build time, tests/pathb/Makefile REF=)")
     for n, size in (("08", 1000), ("05", 1000)):
         out = tmp_path / f"image-{n}.png"
         proc = subprocess.run([str(exe), str(scene_path(f"inputs/input-{n}.rti")), "-o", str(out), "-h", str(size), "-w", str(size),
@@ -445,9 +445,9 @@ def _scene_from_text(pkg, tmp_path, name, text):
 CAM = "cam 0 0 30  -10 -10 10  10 -10 10  -10 10 10  10 10 10\n"
 
 
-def test_empty_and_lightless_scenes(pkg, gpu_renderer, oracle, reference, tmp_path):
+def test_empty_and_lightless_scenes(pkg, gpu_renderer, oracle, live_reference, tmp_path):
     """No geometry at all; geometry without any light; only an ambient light: frames, ids and ray counts equal the
-    oracle's, and the unmodified reference agrees on the frame."""
+    oracle's, and the unmodified reference agrees on the frame where it is built."""
     cases = {
         "nothing.rti": CAM,
         "dark.rti": CAM + "mat 0.1 0.1 0.1 0.5 0.5 0.5 0.3 0.3 0.3 10 0.5 0.5 0.5\nsph 0 0 0 4\n",
@@ -465,9 +465,10 @@ def test_empty_and_lightless_scenes(pkg, gpu_renderer, oracle, reference, tmp_pa
             assert np.array_equal(geom, o_geom) and np.array_equal(face, o_face), name
             assert [st["rays_primary"], st["rays_shadow"], st["rays_secondary"]] == counts[:3], name
             assert np.abs(rgb - o_rgb).max() <= FP64_TOL, name
-        href = reference.load(tmp_path / name)
-        r_rgb, _, _, _ = reference.render(href, 40, 30, 3, threads=2)
-        assert np.abs(gpu_renderer.render(40, 30, 3) - r_rgb).max() <= FP64_TOL, name
+        if live_reference is not None:
+            href = live_reference.load(tmp_path / name)
+            r_rgb, _, _, _ = live_reference.render(href, 40, 30, 3, threads=2)
+            assert np.abs(gpu_renderer.render(40, 30, 3) - r_rgb).max() <= FP64_TOL, name
         img = gpu_renderer.render_rgb8(40, 30, 3)
         assert np.array_equal(img, quantize(gpu_renderer.render(40, 30, 3)))
 
