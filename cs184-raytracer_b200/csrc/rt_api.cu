@@ -594,7 +594,7 @@ int rt_scene_upload(rt_context* ctx, const rt_scene* s) {
         float pad_scale = 0.f;
         CU(ctx->nodes.ensure(n_bvh + 2));
         int brc = build_lbvh(S, ctx->bvh_prims.p, group_first_code, (int)n_bvh, group_sizes, 2, extra_abs, st,
-                             ctx->scratch, ctx->nodes.p, &node_count, &launches, err, sizeof(err), cb, nullptr, &pad_scale);
+                             ctx->scratch, ctx->nodes.p, &node_count, &launches, err, sizeof(err), cb, &pad_scale);
         ctx->scratch.reset();
         if (brc != RT_OK) return fail(brc, "LBVH build: %s", err);
         S.origin_limit = pad_scale;

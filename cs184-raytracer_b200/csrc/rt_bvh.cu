@@ -1,9 +1,10 @@
 // rt_bvh.cu — GPU LBVH build: primitive bounds -> 30-bit Morton codes -> hand-written
 // LSD radix sort (no CUB) -> Karras hierarchy (pure integer, deterministic) -> bottom-up
-// refit -> surface-area-guided collapse into 128-byte 4-wide nodes.  It replaces the reference's only acceleration structure,
+// refit -> treelet restructuring -> least-cost collapse into 128-byte 4-wide nodes.  It replaces the reference's only acceleration structure,
 // one object-space AABB per .obj mesh (Mesh::updateBoundingBox src/geometry.cpp:145-162,
 // hitsBoundingBox src/geometry.cpp:5-29).  The boxes only CULL (FP32, padded outward);
 // every hit decision is still the exact FP64 test in rt_device.cuh.
+#include <algorithm>
 #include <cfloat>
 #include <cmath>
 #include <cstdio>
@@ -183,53 +184,260 @@ __global__ void k_refit(int n, const int* __restrict__ vals, const float* __rest
     }
 }
 
-// depth of every internal node of one tree (root = 0) by walking the parent chain
+// depth of every internal node of one group's tree (root = 0) by walking the parent chain
 __global__ void k_depth(int n, const int* __restrict__ parent_int, int* __restrict__ depth, int* __restrict__ max_depth) {
     int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n - 1) return;
     int d = 0;
     for (int p = parent_int[i]; p >= 0; p = parent_int[p]) d++;
     depth[i] = d;
-    // deepest internal node of the whole forest (bounds the traversal stack, see build_lbvh)
+    // deepest internal node of this group's tree (bounds the traversal stack of the even-depth collapse, see build_lbvh)
     const unsigned act = __activemask();
     const int m = __reduce_max_sync(act, d);
     if ((int)(threadIdx.x & 31) == __ffs(act) - 1) atomicMax(max_depth, m);
 }
 
-// Surface-area-guided choice of the children of the 4-wide nodes (one launch per level of the wide tree, top down):
-// a binary node that is the root of a wide node in wave w starts from its two children and twice replaces the
-// internal child of LARGEST surface area by that child's two children — the child a ray is most likely to enter
-// anyway is the one whose box test is worth saving — and the internal children that remain become the roots of wave
-// w + 1.  wave_of[]: wave of every root (-1: not a root); slots4[]: the four chosen children (BVH_DONE: none).
-// Against pulling up the grandchildren of every even-depth node: 3.3 % fewer node visits per ray on the 1 M-triangle
-// scene (19.27 -> 18.64 closest hit, 13.28 -> 12.83 any hit).
+// ---- Cost model of the tree optimisations below ----------------------------------------------------------------
+// Surface-area heuristic: a ray that enters a box of area A_parent enters a child box of area A with probability
+// A / A_parent.  The expected work of a ray is then C_node * sum(area of the wide nodes it may visit) + C_prim *
+// sum(area of the leaf boxes), over the area of the root.  The traversal kernels are bound by the LSU write-back of
+// what they load (DESIGN section 5): a wide-node visit loads 112 B, an exact face test 80 B, so C_prim / C_node is
+// about 0.7.  With ONE primitive per leaf the leaf term is the same for every topology over the same primitives, so
+// neither pass below depends on the two constants: the treelet pass minimises the summed area of the binary internal
+// nodes, the collapse the summed area of the binary nodes chosen to be wide nodes.
+__device__ __forceinline__ float box_area(const float* lo, const float* hi) {
+    const float ex = hi[0] - lo[0], ey = hi[1] - lo[1], ez = hi[2] - lo[2];
+    return ex * ey + ey * ez + ez * ex;
+}
+
+// Box of a binary-tree child reference (>= 0 internal node, < 0 leaf ~sorted position), read through L2: the
+// bottom-up passes read what other threads of the same launch wrote.
+__device__ __forceinline__ void child_box(int c, const int* vals, const float* plo, const float* phi, const float* ilo,
+                                          const float* ihi, float lo[3], float hi[3]) {
+    const float *bl, *bh;
+    if (c < 0) {
+        const int p = vals[~c];
+        bl = plo + 3 * (size_t)p; bh = phi + 3 * (size_t)p;
+    } else {
+        bl = ilo + 3 * (size_t)c; bh = ihi + 3 * (size_t)c;
+    }
+    for (int a = 0; a < 3; a++) { lo[a] = __ldcg(bl + a); hi[a] = __ldcg(bh + a); }
+}
+
+// Treelet restructuring (Karras & Aila, HPG 2013), one bottom-up pass with k_refit's arrival counters.  The thread
+// that arrives second at an internal node (both subtrees are final) grows a treelet from it by expanding the
+// internal treelet leaf of largest area until TREELET_LEAVES leaves, finds the topology of least summed internal area
+// over those leaves by dynamic programming over their subsets, and rewires the treelet's own internal nodes into it
+// (the node keeps its index and its parent, so the set of internal indices and the root stay as k_karras made them).
+// Deterministic: every comparison is strict in a fixed order (ties keep the lower slot / the first partition
+// enumerated) and the boxes are min/max of primitive boxes, so scheduling cannot change the result.
+#define TREELET_LEAVES 7
+// Rounds of the whole pass (a later round sees the treelets the earlier one made).  Box tests per frame of the
+// 1 M-triangle scene after 0 / 1 / 2 / 3 rounds (with the least-cost collapse): 24.75 / 23.34 / 22.94 / 22.81 G.
+#define TREELET_ROUNDS 2
+#define TREELET_THREADS 64
+#define COST(s) s_cost[(s) * TREELET_THREADS + threadIdx.x]
+
+// Best split of treelet subset s (>= 2 leaves) into two parts, the part with the lowest leaf returned; each
+// partition is enumerated once, in a fixed order, and the first of equal costs wins.
+__device__ __forceinline__ int treelet_split(const float* s_cost, int s, float* best_cost) {
+    const int low = s & -s, rest = s ^ low;
+    float best = FLT_MAX;
+    int bp = low;
+    for (int q = (rest - 1) & rest;; q = (q - 1) & rest) {
+        const int p = q | low;
+        const float c = COST(p) + COST(s ^ p);
+        if (c < best) { best = c; bp = p; }
+        if (q == 0) break;
+    }
+    *best_cost = best;
+    return bp;
+}
+
+// Launched with TREELET_THREADS threads per block and TREELET_THREADS << TREELET_LEAVES floats of shared memory.
+__global__ void __launch_bounds__(TREELET_THREADS, 1) k_treelet(int n, const int* __restrict__ vals, const float* __restrict__ plo, const float* __restrict__ phi,
+                          int* left, int* right, int* parent_int, int* parent_leaf, float* ilo, float* ihi,
+                          int* __restrict__ flags) {
+    extern __shared__ float s_cost[];
+    int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    int cur = __ldcg(parent_leaf + i);
+    while (cur >= 0) {
+        if (atomicAdd(&flags[cur], 1) == 0) return;
+        __threadfence();
+        int leaf[TREELET_LEAVES], inner[TREELET_LEAVES - 1];
+        float llo[TREELET_LEAVES][3], lhi[TREELET_LEAVES][3], larea[TREELET_LEAVES];
+        int nl = 2, ni = 1;
+        inner[0] = cur;
+        leaf[0] = __ldcg(left + cur);
+        leaf[1] = __ldcg(right + cur);
+        float old_cost;
+        {
+            float lo[3], hi[3];
+            child_box(cur, vals, plo, phi, ilo, ihi, lo, hi);
+            old_cost = box_area(lo, hi);
+        }
+        for (int k = 0; k < 2; k++) {
+            child_box(leaf[k], vals, plo, phi, ilo, ihi, llo[k], lhi[k]);
+            larea[k] = box_area(llo[k], lhi[k]);
+        }
+        while (nl < TREELET_LEAVES) {
+            int best = -1;
+            float ba = -1.f;
+            for (int k = 0; k < nl; k++)
+                if (leaf[k] >= 0 && larea[k] > ba) { ba = larea[k]; best = k; }
+            if (best < 0) break;
+            const int c = leaf[best];
+            inner[ni++] = c;
+            old_cost += ba;
+            leaf[best] = __ldcg(left + c);
+            leaf[nl] = __ldcg(right + c);
+            for (int t = 0; t < 2; t++) {
+                const int k = t ? nl : best;
+                child_box(leaf[k], vals, plo, phi, ilo, ihi, llo[k], lhi[k]);
+                larea[k] = box_area(llo[k], lhi[k]);
+            }
+            nl++;
+        }
+        if (nl > 2) {
+            // COST(s): least summed area of the internal nodes of a tree over the leaves in subset s, in shared memory
+            // as [subset][thread] so that every lane reads its own bank whatever subsets the lanes look up
+            const int full = (1 << nl) - 1;
+            for (int s = 1; s <= full; s++) {
+                if ((s & (s - 1)) == 0) { COST(s) = 0.f; continue; }
+                float lo[3] = {FLT_MAX, FLT_MAX, FLT_MAX}, hi[3] = {-FLT_MAX, -FLT_MAX, -FLT_MAX};
+                for (int k = 0; k < nl; k++)
+                    if (s >> k & 1)
+                        for (int a = 0; a < 3; a++) { lo[a] = fminf(lo[a], llo[k][a]); hi[a] = fmaxf(hi[a], lhi[k][a]); }
+                float best;
+                treelet_split(s_cost, s, &best);
+                COST(s) = box_area(lo, hi) + best;
+            }
+            if (COST(full) < 0.9999f * old_cost) {      // not for a rounding difference of the same topology
+                // rewire: subsets in creation order take the treelet's internal nodes, inner[0] (= cur) stays the root
+                int stack_s[TREELET_LEAVES], stack_n[TREELET_LEAVES], sp = 0, next = 1;
+                stack_s[sp] = full; stack_n[sp++] = cur;
+                while (sp > 0) {
+                    const int s = stack_s[--sp], node = stack_n[sp];
+                    float unused;
+                    const int p = treelet_split(s_cost, s, &unused);
+                    const int part[2] = {p, s ^ p};
+                    int ch[2];
+                    for (int k = 0; k < 2; k++) {
+                        const int q = part[k];
+                        if ((q & (q - 1)) == 0) {
+                            ch[k] = leaf[__ffs(q) - 1];
+                            if (ch[k] < 0) parent_leaf[~ch[k]] = node; else parent_int[ch[k]] = node;
+                        } else {
+                            ch[k] = inner[next++];
+                            parent_int[ch[k]] = node;
+                            stack_s[sp] = q; stack_n[sp++] = ch[k];
+                        }
+                    }
+                    left[node] = ch[0];
+                    right[node] = ch[1];
+                    if (node != cur) {                       // the root's box is the union of the same leaves
+                        float lo[3] = {FLT_MAX, FLT_MAX, FLT_MAX}, hi[3] = {-FLT_MAX, -FLT_MAX, -FLT_MAX};
+                        for (int k = 0; k < nl; k++)
+                            if (s >> k & 1)
+                                for (int a = 0; a < 3; a++) { lo[a] = fminf(lo[a], llo[k][a]); hi[a] = fmaxf(hi[a], lhi[k][a]); }
+                        for (int a = 0; a < 3; a++) { ilo[3 * (size_t)node + a] = lo[a]; ihi[3 * (size_t)node + a] = hi[a]; }
+                    }
+                }
+            }
+        }
+        __threadfence();
+        cur = __ldcg(parent_int + cur);
+    }
+}
+
+// Least-cost collapse of the binary tree into a 4-wide one (Ylitie, Karras & Laine, HPG 2017, section 3), bottom-up
+// with arrival counters.  Per internal node n (areas only, see the cost model above; leaves cost nothing):
+//   S(n, k)  least cost of n's subtree spread over at most k >= 2 slots of the wide node above it without a node for
+//            n itself: min over i + j <= k of D(left, i) + D(right, j);
+//   D(n, 1)  = area(n) + S(n, 4): n becomes a wide node (its four slots hold S(n, 4));
+//   D(n, k)  = min(D(n, 1), S(n, k)) for k = 2..4.
+// dcost[n] = D(n, 1..4); choice[n] packs, for k = 2..4, the split (i | j << 2) of S(n, k) in bits 4(k-2).. and in bit
+// 12 + k whether D(n, k) is n itself.  Ties keep the first candidate in a fixed order: deterministic.
+// wdepth[n] packs, in byte k - 1, the number of wide levels the choice behind D(n, k) puts on the deepest path of n's
+// subtree (saturated at 255), so byte 0 of the root is the depth of the wide tree before any of it is written.
+__global__ void k_collapse_cost(int n, const int* __restrict__ left, const int* __restrict__ right,
+                                const int* __restrict__ parent_int, const int* __restrict__ parent_leaf,
+                                const float* __restrict__ ilo, const float* __restrict__ ihi, float4* dcost,
+                                int* __restrict__ choice, int* wdepth, int* __restrict__ flags) {
+    int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    int cur = parent_leaf[i];
+    while (cur >= 0) {
+        if (atomicAdd(&flags[cur], 1) == 0) return;
+        __threadfence();
+        float dl[5] = {0.f, 0.f, 0.f, 0.f, 0.f}, dr[5] = {0.f, 0.f, 0.f, 0.f, 0.f};
+        const int l = left[cur], r = right[cur];
+        if (l >= 0) { const float4 d = __ldcg(dcost + l); dl[1] = d.x; dl[2] = d.y; dl[3] = d.z; dl[4] = d.w; }
+        if (r >= 0) { const float4 d = __ldcg(dcost + r); dr[1] = d.x; dr[2] = d.y; dr[3] = d.z; dr[4] = d.w; }
+        int wl[5] = {0, 0, 0, 0, 0}, wr[5] = {0, 0, 0, 0, 0};
+        if (l >= 0) { const int w = __ldcg(wdepth + l); for (int k = 1; k <= 4; k++) wl[k] = w >> (8 * (k - 1)) & 255; }
+        if (r >= 0) { const int w = __ldcg(wdepth + r); for (int k = 1; k <= 4; k++) wr[k] = w >> (8 * (k - 1)) & 255; }
+        float s[5];
+        int ws[5];                                // wide levels below the slots of S(n, k)
+        int code = 0, sij = 1 | 1 << 2;
+        s[2] = dl[1] + dr[1];
+        ws[2] = max(wl[1], wr[1]);
+        for (int k = 2; k <= 4; k++) {
+            if (k > 2) { s[k] = s[k - 1]; ws[k] = ws[k - 1]; }
+            for (int a = 1; a < k; a++) {
+                const float c = dl[a] + dr[k - a];
+                if (c < s[k]) { s[k] = c; sij = a | (k - a) << 2; ws[k] = max(wl[a], wr[k - a]); }
+            }
+            code |= sij << (4 * (k - 2));
+        }
+        float lo[3], hi[3];
+        for (int a = 0; a < 3; a++) { lo[a] = ilo[3 * (size_t)cur + a]; hi[a] = ihi[3 * (size_t)cur + a]; }
+        float d[5];
+        d[1] = box_area(lo, hi) + s[4];
+        const int w1 = min(ws[4] + 1, 255);
+        int wd = w1;
+        for (int k = 2; k <= 4; k++) {
+            if (d[1] <= s[k]) { d[k] = d[1]; code |= 1 << (12 + k); wd |= w1 << (8 * (k - 1)); }
+            else { d[k] = s[k]; wd |= ws[k] << (8 * (k - 1)); }
+        }
+        dcost[cur] = make_float4(d[1], d[2], d[3], d[4]);
+        choice[cur] = code;
+        wdepth[cur] = wd;
+        __threadfence();
+        cur = parent_int[cur];
+    }
+}
+
+// Top-down half of the collapse, one launch per level of the wide tree: every wide node of wave w expands its S(n, 4)
+// into at most four slots; the internal nodes among them are the wide nodes of wave w + 1.  wave_of[]: wave of every
+// wide node (-1: none); slots4[]: its children (BVH_DONE: none).
 __global__ void k_choose_children(int n, int wave, int* __restrict__ wave_of, int4* __restrict__ slots4,
                                   const int* __restrict__ left, const int* __restrict__ right,
-                                  const float* __restrict__ ilo, const float* __restrict__ ihi, int* __restrict__ wave_any) {
+                                  const int* __restrict__ choice) {
     int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n - 1 || wave_of[i] != wave) return;
-    int slots[4] = {left[i], right[i], BVH_DONE, BVH_DONE};
-    int ns = 2;
-    for (int rep = 0; rep < 2; rep++) {
-        int best = -1;
-        float best_area = -1.f;
-        for (int k = 0; k < ns; k++) {
-            if (slots[k] < 0) continue;
-            const float* bl = ilo + 3 * (size_t)slots[k];
-            const float* bh = ihi + 3 * (size_t)slots[k];
-            const float ex = bh[0] - bl[0], ey = bh[1] - bl[1], ez = bh[2] - bl[2];
-            const float area = ex * ey + ey * ez + ez * ex;
-            if (area > best_area) { best_area = area; best = k; }
-        }
-        if (best < 0) break;
-        const int c = slots[best];
-        slots[best] = left[c];
-        slots[ns++] = right[c];
+    int slots[4] = {BVH_DONE, BVH_DONE, BVH_DONE, BVH_DONE};
+    int ns = 0;
+    int st_n[4], st_k[4], sp = 0;                // (subtree, slots it may fill); at most four entries are pending
+    {
+        const int ij = choice[i] >> 8 & 15;      // split of S(i, 4)
+        st_n[sp] = right[i]; st_k[sp++] = ij >> 2;
+        st_n[sp] = left[i]; st_k[sp++] = ij & 3;
     }
-    for (int k = 0; k < ns; k++)
-        if (slots[k] >= 0) wave_of[slots[k]] = wave + 1;
+    while (sp > 0) {
+        const int c = st_n[--sp], k = st_k[sp];
+        const int code = c >= 0 ? choice[c] : 0;
+        if (c < 0 || k == 1 || (code >> (12 + k) & 1)) {
+            slots[ns++] = c;
+            if (c >= 0) wave_of[c] = wave + 1;
+            continue;
+        }
+        const int ij = code >> (4 * (k - 2)) & 15;
+        st_n[sp] = right[c]; st_k[sp++] = ij >> 2;
+        st_n[sp] = left[c]; st_k[sp++] = ij & 3;
+    }
     slots4[i] = make_int4(slots[0], slots[1], slots[2], slots[3]);
-    wave_any[wave] = 1;          // same value from every root of the wave: the deepest marked wave is the wide tree's depth
 }
 
 // Binary Karras nodes at EVEN depth become 4-wide nodes: each internal child (odd depth) is
@@ -299,7 +507,6 @@ __global__ void k_pack_wide(int n, const int* __restrict__ vals, const int* __re
     nodes[node_offset + i] = nd;
 }
 
-#define RT_MAX_WAVES 256      // levels of the wide tree k_choose_children may walk (the traversal stack allows far fewer)
 #define TAKE(var, type, count)                                                         \
     do {                                                                               \
         var = arena.take<type>((size_t)(count));                                       \
@@ -323,21 +530,18 @@ __global__ void k_pack_wide(int n, const int* __restrict__ vals, const int* __re
 // otherwise stretch the leaf-level boxes of the mesh over the whole air space.
 int build_lbvh(const DScene& S, const int* d_codes, const int* group_first_code, int n, const int* group_sizes, int ngroups,
                float extra_abs, cudaStream_t stream, DeviceArena& arena, BvhNode* nodes, size_t* out_count,
-               int* launches, char* err, int errlen, float* centroid_bounds, int* out_max_depth, float* out_pad_scale) {
+               int* launches, char* err, int errlen, float* centroid_bounds, float* out_pad_scale) {
     *out_count = 0;
     float *plo = nullptr, *phi = nullptr, *ilo = nullptr, *ihi = nullptr;
     int *gb = nullptr, *vals0 = nullptr, *vals1 = nullptr, *hist = nullptr;
     int4* slots4 = nullptr;
-    int* wave_any = nullptr;
-    std::vector<int> h_wave_any(RT_MAX_WAVES, 0);
     int *left = nullptr, *right = nullptr, *pint = nullptr, *pleaf = nullptr, *flags = nullptr, *depth = nullptr;
     uint32_t *keys0 = nullptr, *keys1 = nullptr;
     const int T = 256;
     const int nblk = (n + T - 1) / T;
+    float4* dcost = nullptr;
+    int *choice = nullptr, *wdepth = nullptr;
     int hb[7];
-    int max_bin_depth = 0, max_wide_wave = 0;
-    // RT_LBVH_COLLAPSE=even: round 1's fixed collapse (every even-depth binary node pulls up its grandchildren), for A/B
-    const bool sah_collapse = !(getenv("RT_LBVH_COLLAPSE") && !strcmp(getenv("RT_LBVH_COLLAPSE"), "even"));
     float pad_scale = 0.f;
     struct Group { int start, n, root_ref, first_code; float box[6]; };
     Group groups[4];
@@ -389,9 +593,9 @@ int build_lbvh(const DScene& S, const int* d_codes, const int* group_first_code,
         TAKE(ilo, float, 3 * (size_t)n);
         TAKE(ihi, float, 3 * (size_t)n);
         TAKE(slots4, int4, (size_t)n);
-        TAKE(wave_any, int, RT_MAX_WAVES);
-        CK(cudaMemsetAsync(wave_any, 0, sizeof(int) * RT_MAX_WAVES, stream));
-        CK(cudaMemsetAsync(flags, 0, sizeof(int) * (size_t)n, stream));
+        TAKE(dcost, float4, (size_t)n);
+        TAKE(choice, int, (size_t)n);
+        TAKE(wdepth, int, (size_t)n);
         k_morton<<<nblk, T, 0, stream>>>(plo, phi, n, gb, keys0, vals0);
         (*launches)++;
         size_t node_cursor = (size_t)nsuper;
@@ -409,54 +613,74 @@ int build_lbvh(const DScene& S, const int* d_codes, const int* group_first_code,
             int *vin = vals0 + gs, *vout = vals1 + gs;
             sort_pairs(stream, kin, kout, vin, vout, hist, gn, nullptr, 32, launches);
             // kin/vin now point at the sorted data
-            k_karras<<<gblk, T, 0, stream>>>(kin, gn, left + gs, right + gs, pint + gs, pleaf + gs);
-            k_refit<<<gblk, T, 0, stream>>>(gn, vin, plo, phi, left + gs, right + gs, pint + gs, pleaf + gs,
-                                            ilo + 3 * (size_t)gs, ihi + 3 * (size_t)gs, flags + gs);
-            k_depth<<<gblk, T, 0, stream>>>(gn, pint + gs, depth + gs, gb + 7);
-            if (!sah_collapse) {
-                k_pack_wide<<<gblk, T, 0, stream>>>(gn, vin, d_codes, plo, phi, left + gs, right + gs, ilo + 3 * (size_t)gs,
-                                                    ihi + 3 * (size_t)gs, depth + gs, gb, nodes, (int)node_cursor, nullptr, nullptr);
-            } else {
-                // one light launch per level of the wide tree; the wide tree is at most as deep as the binary one
+            float *gilo = ilo + 3 * (size_t)gs, *gihi = ihi + 3 * (size_t)gs;
+            int *gleft = left + gs, *gright = right + gs, *gpint = pint + gs, *gpleaf = pleaf + gs, *gflags = flags + gs;
+            const size_t flag_bytes = sizeof(int) * (size_t)gn;
+            // The optimised build (treelets + least-cost collapse) can be deeper than the traversal stack allows where
+            // the Karras tree is not; then the group is built again as a plain Karras tree with the even-depth
+            // collapse, whose wide depth is half the binary depth.
+            for (int optimised = 1; optimised >= 0; optimised--) {
+                k_karras<<<gblk, T, 0, stream>>>(kin, gn, gleft, gright, gpint, gpleaf);
+                CK(cudaMemsetAsync(gflags, 0, flag_bytes, stream));
+                k_refit<<<gblk, T, 0, stream>>>(gn, vin, plo, phi, gleft, gright, gpint, gpleaf, gilo, gihi, gflags);
+                (*launches) += 2;
+                if (optimised)
+                    for (int r = 0; r < TREELET_ROUNDS; r++) {
+                        CK(cudaMemsetAsync(gflags, 0, flag_bytes, stream));
+                        k_treelet<<<(gn + TREELET_THREADS - 1) / TREELET_THREADS, TREELET_THREADS,
+                                    sizeof(float) * (TREELET_THREADS << TREELET_LEAVES), stream>>>(gn, vin, plo, phi, gleft, gright, gpint, gpleaf, gilo, gihi, gflags);
+                        (*launches)++;
+                    }
+                // The traversal defers at most 3 siblings per wide level; the stack (RT_SH_STACK shared + RT_STACK
+                // local entries) must hold them all on every root-to-leaf path (+ the super node), or the build
+                // fails instead of silently dropping subtrees.
+                const int stack_entries = RT_STACK + RT_SH_STACK;
+                int* wave_of = gflags;
+                if (optimised) {
+                    CK(cudaMemsetAsync(gflags, 0, flag_bytes, stream));
+                    k_collapse_cost<<<gblk, T, 0, stream>>>(gn, gleft, gright, gpint, gpleaf, gilo, gihi, dcost + gs,
+                                                            choice + gs, wdepth + gs, gflags);
+                    (*launches)++;
+                    int wide_depth = 0;
+                    CK(cudaMemcpyAsync(&wide_depth, wdepth + gs, sizeof(int), cudaMemcpyDeviceToHost, stream));
+                    CK(cudaStreamSynchronize(stream));
+                    wide_depth &= 255;                  // D(root, 1): the group's root is a wide node
+                    if (3 * (wide_depth + nsuper) > stack_entries) continue;
+                    // one light launch per level of the wide tree
+                    CK(cudaMemsetAsync(wave_of, 0xff, flag_bytes, stream));
+                    CK(cudaMemsetAsync(wave_of, 0, sizeof(int), stream));                      // the group's root: wave 0
+                    for (int w = 0; w < wide_depth; w++) {
+                        k_choose_children<<<gblk, T, 0, stream>>>(gn, w, wave_of, slots4 + gs, gleft, gright, choice + gs);
+                        (*launches)++;
+                    }
+                    k_pack_wide<<<gblk, T, 0, stream>>>(gn, vin, d_codes, plo, phi, gleft, gright, gilo, gihi, nullptr, gb,
+                                                        nodes, (int)node_cursor, wave_of, slots4 + gs);
+                    (*launches)++;
+                    break;
+                }
+                CK(cudaMemsetAsync(gb + 7, 0, sizeof(int), stream));
+                k_depth<<<gblk, T, 0, stream>>>(gn, gpint, depth + gs, gb + 7);
+                (*launches)++;
                 int gdepth = 0;
                 CK(cudaMemcpyAsync(&gdepth, gb + 7, sizeof(int), cudaMemcpyDeviceToHost, stream));
                 CK(cudaStreamSynchronize(stream));
-                int* wave_of = flags + gs;            // k_refit is done with its arrival counters
-                CK(cudaMemsetAsync(wave_of, 0xff, sizeof(int) * (size_t)gn, stream));
-                CK(cudaMemsetAsync(wave_of, 0, sizeof(int), stream));                          // the group's root: wave 0
-                if (gdepth + 1 > RT_MAX_WAVES) gdepth = RT_MAX_WAVES - 1;      // deeper trees fail the stack check below anyway
-                for (int w = 0; w <= gdepth; w++) {
-                    k_choose_children<<<gblk, T, 0, stream>>>(gn, w, wave_of, slots4 + gs, left + gs, right + gs, ilo + 3 * (size_t)gs,
-                                                              ihi + 3 * (size_t)gs, wave_any);
-                    (*launches)++;
+                const int wide_levels = gdepth / 2 + 1 + nsuper;
+                if (3 * wide_levels > stack_entries) {
+                    snprintf(err, errlen, "LBVH is %d binary levels deep: %d deferred entries exceed the traversal stack of %d",
+                             gdepth + 1, 3 * wide_levels, stack_entries);
+                    return RT_ERR_LIMIT;
                 }
-                k_pack_wide<<<gblk, T, 0, stream>>>(gn, vin, d_codes, plo, phi, left + gs, right + gs, ilo + 3 * (size_t)gs,
-                                                    ihi + 3 * (size_t)gs, depth + gs, gb, nodes, (int)node_cursor, wave_of, slots4 + gs);
+                k_pack_wide<<<gblk, T, 0, stream>>>(gn, vin, d_codes, plo, phi, gleft, gright, gilo, gihi, depth + gs, gb,
+                                                    nodes, (int)node_cursor, nullptr, nullptr);
+                (*launches)++;
             }
-            (*launches) += 4;
             groups[g].root_ref = (int)node_cursor;
             CK(cudaMemcpyAsync(groups[g].box, ilo + 3 * (size_t)gs, 12, cudaMemcpyDeviceToHost, stream));
             CK(cudaMemcpyAsync(groups[g].box + 3, ihi + 3 * (size_t)gs, 12, cudaMemcpyDeviceToHost, stream));
             node_cursor += (size_t)(gn - 1);
         }
-        CK(cudaMemcpyAsync(&max_bin_depth, gb + 7, sizeof(int), cudaMemcpyDeviceToHost, stream));
-        CK(cudaMemcpyAsync(h_wave_any.data(), wave_any, sizeof(int) * RT_MAX_WAVES, cudaMemcpyDeviceToHost, stream));
         CK(cudaStreamSynchronize(stream));
         CK(cudaGetLastError());
-        for (int w = 0; w < RT_MAX_WAVES; w++)
-            if (h_wave_any[(size_t)w]) max_wide_wave = w;
-        {   // The traversal defers at most 3 siblings per wide level.  Wide levels on a root-to-leaf path: one per
-            // two binary levels (even-depth collapse) + the super node.  The stack (RT_SH_STACK shared + RT_STACK
-            // local entries) must hold them all; Karras trees over 30-bit codes with index-split duplicates stay
-            // far below this, so a scene that does not is rejected instead of silently dropping subtrees.
-            const int wide_levels = (sah_collapse ? max_wide_wave + 1 : max_bin_depth / 2 + 1) + nsuper;
-            if (3 * wide_levels > RT_STACK + RT_SH_STACK) {
-                snprintf(err, errlen, "LBVH is %d binary levels deep: %d deferred entries exceed the traversal stack of %d",
-                         max_bin_depth + 1, 3 * wide_levels, RT_STACK + RT_SH_STACK);
-                return RT_ERR_LIMIT;
-            }
-            if (out_max_depth) *out_max_depth = max_bin_depth;
-        }
         if (nsuper > 0) {
             const float pad = 2e-6f * fmaxf(pad_scale, 1e-30f);
             float lo[3][4], hi[3][4];

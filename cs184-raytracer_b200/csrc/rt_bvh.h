@@ -35,7 +35,7 @@ struct DeviceArena {
 
 // scratch bytes build_lbvh takes from the arena for n primitives
 inline size_t lbvh_scratch_bytes(size_t n) {
-    return 4 * DeviceArena::padded(12 * n) + 10 * DeviceArena::padded(4 * n) + DeviceArena::padded(16 * n) + DeviceArena::padded(4 * 256) + DeviceArena::padded(4 * 256 * 4097 /* radix-sort histograms, SORT_MAX_BLOCKS + 1 */) + 4096;
+    return 4 * DeviceArena::padded(12 * n) + 12 * DeviceArena::padded(4 * n) + 2 * DeviceArena::padded(16 * n) + DeviceArena::padded(4 * 256 * 4097 /* radix-sort histograms, SORT_MAX_BLOCKS + 1 */) + 4096;
 }
 
 // Builds one LBVH per primitive group over the n primitive codes in d_codes (device;
@@ -48,7 +48,6 @@ int build_lbvh(const DScene& S, const int* d_codes, const int* group_first_code,
                float extra_abs, cudaStream_t stream, DeviceArena& arena, BvhNode* nodes /* >= n + ngroups */,
                size_t* out_count, int* launches, char* err, int errlen,
                float* centroid_bounds /* [6] or null: min xyz, max xyz of the primitive centroids */,
-               int* out_max_depth /* or null: depth of the deepest internal binary node */,
                float* out_pad_scale /* or null: the largest |coordinate| the box padding covers */);
 
 }  // namespace rt
