@@ -611,7 +611,7 @@ int build_lbvh(const DScene& S, const int* d_codes, const int* group_first_code,
             // radix sort of this group's (key, prim index) pairs: 4 passes x 8 bits
             uint32_t *kin = keys0 + gs, *kout = keys1 + gs;
             int *vin = vals0 + gs, *vout = vals1 + gs;
-            sort_pairs(stream, kin, kout, vin, vout, hist, gn, nullptr, 32, launches);
+            sort_pairs(stream, kin, kout, vin, vout, hist, gn, nullptr, launches);
             // kin/vin now point at the sorted data
             float *gilo = ilo + 3 * (size_t)gs, *gihi = ihi + 3 * (size_t)gs;
             int *gleft = left + gs, *gright = right + gs, *gpint = pint + gs, *gpleaf = pleaf + gs, *gflags = flags + gs;

@@ -154,7 +154,6 @@ struct DScene {
     int num_all;
     int num_bvh_prims;
     int single_leaf;           // BVH with exactly one primitive: its prim code
-    int shadow_mode;           // bit 0: light-major thread mapping of k_shadow
     // Largest |coordinate| the LBVH box padding was derived for (every primitive's world bounds,
     // flat ones included, and the camera eye): the FP32 slab test is conservative for ray origins
     // inside it.  A ray starting further out (only possible through rt_cast_rays) takes the
@@ -421,9 +420,6 @@ __device__ __forceinline__ void slab1(const FRay& r, float nx, float ny, float n
 }
 
 #define RT_STACK 96
-#ifndef RT_ANYHIT_UNSORTED
-#define RT_ANYHIT_UNSORTED 1
-#endif
 // Entries of the traversal stack kept in SHARED memory per thread (interleaved by thread, so
 // any mix of stack depths within a warp is bank-conflict free); deeper entries overflow to
 // the local-memory array.  ncu (round 1): with the whole stack in local memory, local
@@ -543,7 +539,7 @@ __device__ __forceinline__ void descend(const DScene& S, const FRay& fr, float t
         slab1(fr, nx.y, ny.y, nz.y, fx.y, fy.y, fz.y, tlim, t1, h1);
         slab1(fr, nx.z, ny.z, nz.z, fx.z, fy.z, fz.z, tlim, t2, h2);
         slab1(fr, nx.w, ny.w, nz.w, fx.w, fy.w, fz.w, tlim, t3, h3);
-        if (ANYHIT && RT_ANYHIT_UNSORTED) {
+        if (ANYHIT) {
             // occlusion query: any order will do; take the first hit slot, defer the others
             int next = h3 ? ref.w : BVH_DONE;
             if (st.roomy(3)) {

@@ -26,7 +26,7 @@ namespace rt {
 #ifndef RT_SHADOW_MINBLOCKS
 #define RT_SHADOW_MINBLOCKS 16
 #endif
-// Light-major tile of k_shadow (hits); 0 = one tile spanning the whole hit queue.
+// Light-major tile of k_shadow (hits).
 #ifndef RT_SHADOW_TILE
 #define RT_SHADOW_TILE 4096
 #endif
@@ -54,14 +54,18 @@ struct HitQ {
     __device__ __forceinline__ double& fld(int k, size_t i) const { return f[(size_t)k * cap + i]; }
 };
 
-// device counters
+// Device counters of one bounce level: a block of CTR_COUNT words that starts half-way into a 128-byte
+// L2 line.  CTR_HITS, CTR_NEXT, CTR_NEXT_T are reset and read back per chunk as one range, with a line
+// boundary between CTR_NEXT and CTR_NEXT_T: every warp of k_shade appends to both, and the appends are
+// slower when the two share a line (B200 at 1000 W, 8K synthetic frame: k_shade 7.46 ms on two lines, 8.0 ms on one).
 enum {
-    CTR_HITS = 0, CTR_NEXT = 1, CTR_DEGENERATE = 2,
-    CTR_NODES = 3, CTR_TRIS = 4, CTR_SPHERES = 5,          // closest-hit kernel
-    CTR_S_NODES = 6, CTR_S_TRIS = 7, CTR_S_SPHERES = 8,    // shadow kernel
-    CTR_NEXT_T = 9,                                        // refracted children (stored from the END of the next queue)
-    CTR_S_CULLED = 10,                                     // shadow rays answered without a traversal (COUNT builds)
-    CTR_COUNT = 12
+    CTR_DEGENERATE = 0,
+    CTR_S_CULLED = 1,                                      // shadow rays answered without a traversal (COUNT builds)
+    CTR_NODES = 2, CTR_TRIS = 3, CTR_SPHERES = 4,          // closest-hit kernel
+    CTR_HITS = 6, CTR_NEXT = 7,                            // the last two words of the first line
+    CTR_NEXT_T = 8,                                        // refracted children (stored from the END of the next queue)
+    CTR_S_NODES = 9, CTR_S_TRIS = 10, CTR_S_SPHERES = 11,  // shadow kernel
+    CTR_COUNT = 16                                         // 128 bytes: every block straddles a line boundary the same way
 };
 
 struct FrameInfo {
@@ -182,7 +186,7 @@ __global__ void __launch_bounds__(RT_BLOCK, RT_TRACE_MINBLOCKS) k_trace(DScene S
     double w0 = 1.0;
     int meta = 0, pixel = -1;
     if (PRIMARY) {
-        if (active) pixel = primary_ray(S, pr, t, o, d, w0);
+        if (active) pixel = primary_ray(S, pr, (int)g, o, d, w0);
         meta = pr.depth;
     } else {
         pixel = active ? q.pixel[i] : -1;
@@ -223,7 +227,6 @@ __global__ void __launch_bounds__(RT_BLOCK, RT_TRACE_MINBLOCKS) k_trace(DScene S
 struct SortGrid {
     float lo[3];
     float scale;      // cells per world unit (same on the three axes: cubic cells)
-    int bits;         // key bits (multiple of 8 for the radix passes)
 };
 __device__ __forceinline__ uint32_t spread_bits3(uint32_t v) {   // 10 bits -> every third bit
     v = (v * 0x00010001u) & 0xFF0000FFu;
@@ -242,8 +245,7 @@ __global__ void k_hit_keys(HitQ h, const unsigned long long* __restrict__ lc, So
         float u = (p[a] - g.lo[a]) * g.scale;
         q[a] = (uint32_t)min(max((int)u, 0), 1023);
     }
-    const uint32_t m = (spread_bits3(q[0]) << 2) | (spread_bits3(q[1]) << 1) | spread_bits3(q[2]);
-    keys[j] = g.bits < 30 ? m >> (30 - g.bits) : m;     // the top `bits` bits: coarser cells, fewer radix passes
+    keys[j] = (spread_bits3(q[0]) << 2) | (spread_bits3(q[1]) << 1) | spread_bits3(q[2]);
     vals[j] = (int)j;
 }
 // --intersection-only: pixel = 1/dist^2 on all channels (src/scene.cpp:69-70)
@@ -394,23 +396,16 @@ __global__ void __launch_bounds__(RT_BLOCK, RT_SHADOW_MINBLOCKS) k_shadow(DScene
     if (t < nhits * nsl) {
         // light-major mapping: a warp = 32 consecutive hits (neighbouring pixels) towards the
         // SAME light, so its shadow rays are coherent; hit-record loads coalesce
-        unsigned li, j;
-        if (S.shadow_mode & 1) {
-#if RT_SHADOW_TILE > 0
-            // ... in tiles of RT_SHADOW_TILE hits: all lights of one tile are processed back to
-            // back, so its hit records (116 B each) are fetched from DRAM once and re-read from
-            // L2 by the other lights instead of streaming the whole queue once per light
-            unsigned long long tile;
-            if (nhits * nsl <= 0xffffffffull) tile = (unsigned)t / (RT_SHADOW_TILE * nsl);     // 32-bit divide: ~5x cheaper
-            else tile = t / ((unsigned long long)RT_SHADOW_TILE * nsl);
-            const unsigned long long first = tile * RT_SHADOW_TILE;
-            const unsigned w = (unsigned)min((unsigned long long)RT_SHADOW_TILE, nhits - first);   // hits in this tile
-            const unsigned r = (unsigned)(t - tile * RT_SHADOW_TILE * nsl);
-            li = r / w; j = (unsigned)first + r % w;
-#else
-            li = (unsigned)(t / nhits); j = (unsigned)(t % nhits);
-#endif
-        } else { j = (unsigned)(t / nsl); li = (unsigned)(t % nsl); }
+        // ... in tiles of RT_SHADOW_TILE hits: all lights of one tile are processed back to
+        // back, so its hit records (116 B each) are fetched from DRAM once and re-read from
+        // L2 by the other lights instead of streaming the whole queue once per light
+        unsigned long long tile;
+        if (nhits * nsl <= 0xffffffffull) tile = (unsigned)t / (RT_SHADOW_TILE * nsl);     // 32-bit divide: ~5x cheaper
+        else tile = t / ((unsigned long long)RT_SHADOW_TILE * nsl);
+        const unsigned long long first = tile * RT_SHADOW_TILE;
+        const unsigned w = (unsigned)min((unsigned long long)RT_SHADOW_TILE, nhits - first);   // hits in this tile
+        const unsigned r = (unsigned)(t - tile * RT_SHADOW_TILE * nsl);
+        const unsigned li = r / w, j = (unsigned)first + r % w;
         const DLight* l = S.slights + li;
         d3 P = mk3(h.fld(0, j), h.fld(1, j), h.fld(2, j));
         d3 N = mk3(h.fld(3, j), h.fld(4, j), h.fld(5, j));

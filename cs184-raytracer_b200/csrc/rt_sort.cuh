@@ -120,15 +120,15 @@ static __global__ void k_sort_scatter(const uint32_t* __restrict__ keys_in, cons
     }
 }
 
-// Sorts by the low `bits` (multiple of 8) key bits.  n_max sizes the grid; the real count is
-// n_max, or *n_dev when n_dev != nullptr.  On return kin/vin point at the sorted data (the
-// pointers are swapped once per pass).  hist: 256 * (SORT_MAX_BLOCKS + 1) ints of scratch.
+// Sorts by all 32 key bits (four passes).  n_max sizes the grid; the real count is n_max, or
+// *n_dev when n_dev != nullptr.  On return kin/vin point at the sorted data (the pointers are
+// swapped once per pass).  hist: 256 * (SORT_MAX_BLOCKS + 1) ints of scratch.
 static inline void sort_pairs(cudaStream_t stream, uint32_t*& kin, uint32_t*& kout, int*& vin, int*& vout, int* hist,
-                              int n_max, const unsigned long long* n_dev, int bits, int* launches) {
+                              int n_max, const unsigned long long* n_dev, int* launches) {
     int sblocks = (n_max + 4095) / 4096;
     if (sblocks > SORT_MAX_BLOCKS) sblocks = SORT_MAX_BLOCKS;
     if (sblocks < 1) sblocks = 1;
-    for (int shift = 0; shift < bits; shift += 8) {
+    for (int shift = 0; shift < 32; shift += 8) {
         k_sort_hist<<<sblocks, SORT_THREADS, 0, stream>>>(kin, n_max, n_dev, shift, sblocks, hist);
         int* totals = hist + (size_t)256 * SORT_MAX_BLOCKS;
         k_sort_rowscan<<<256, SORT_THREADS, 0, stream>>>(hist, sblocks, totals);

@@ -296,14 +296,13 @@ def test_synthetic_scene_lbvh_vs_brute_force(pkg, gpu_renderer):
 
 
 @pytest.mark.parametrize("name", ["input-02", "input-03", "bunny4"])
-@pytest.mark.parametrize("env", [
-    {"RT_HIT_SORT_MIN_RAYS": "1"},                                        # hit sorting on every level
-    {"RT_HIT_SORT_MIN_RAYS": "1", "RT_HIT_SORT_BITS": "8"},               # one radix pass
-    {"RT_HIT_SORT_MIN_RAYS": "1", "RT_QUEUE_CAP": "8192"},                # sorted chunks of a chunked level
-    {"RT_HIT_SORT_BITS": "0"},                                            # sorting off
-    {"RT_NO_OVERLAP": "1", "RT_HIT_SORT_MIN_RAYS": "1"},                  # kernels strictly serial
-], ids=["sort", "sort8", "sort-chunked", "nosort", "serial"])
-def test_hit_sorting_and_overlap_do_not_change_the_result(pkg, scenes, monkeypatch, name, env):
+@pytest.mark.parametrize("env,serial", [
+    ({"RT_HIT_SORT_MIN_RAYS": "1"}, False),                               # hit sorting on every level
+    ({"RT_HIT_SORT_MIN_RAYS": "1", "RT_QUEUE_CAP": "8192"}, False),       # sorted chunks of a chunked level
+    ({"RT_HIT_SORT_MIN_RAYS": str(2**31)}, False),                        # sorting off: no level is that large
+    ({"RT_HIT_SORT_MIN_RAYS": "1"}, True),                                # RT_FLAG_SERIAL: kernels strictly serial
+], ids=["sort", "sort-chunked", "nosort", "serial"])
+def test_hit_sorting_and_overlap_do_not_change_the_result(pkg, scenes, monkeypatch, name, env, serial):
     """The Morton hit sort, the shadow/trace overlap and their thresholds only reorder work: hit ids, ray
     counts and the frame (FP64 sums reorder at 1e-16) must equal the reference outputs."""
     for k, v in env.items():
@@ -313,7 +312,7 @@ def test_hit_sorting_and_overlap_do_not_change_the_result(pkg, scenes, monkeypat
         sc = scenes(name)
         r.upload(sc)
         fx = load_ref_fixture(name, 96, 96)
-        rgb = r.render(96, 96, int(fx["depth"]))
+        rgb = r.render(96, 96, int(fx["depth"]), flags=pkg.RT_FLAG_SERIAL if serial else 0)
         st = r.stats()
         assert st["rays_primary"] + st["rays_shadow"] + st["rays_secondary"] == int(fx["castray_calls"])
         assert np.abs(rgb - fx["rgb"]).max() <= FP64_TOL
