@@ -380,8 +380,11 @@ int rt_scene_upload(rt_context* ctx, const rt_scene* s) {
             double r = std::fmin(1.0, std::fmax(-1.0, detC / 2));
             lmax = q + 2 * p * std::cos(std::acos(r) / 3);
         }
+        // the stored centre is c rounded to FP32: grow the radius by that rounding (sum of the axes >= its length)
+        const float cf[3] = {(float)c[0], (float)c[1], (float)c[2]};
         double rw = std::fabs(g.radius) * std::sqrt(std::fmax(lmax, 0.0)) * (1.0 + 1e-6);
-        hsb[(size_t)i] = make_float4((float)c[0], (float)c[1], (float)c[2], std::nextafter((float)rw, INFINITY));
+        for (int a = 0; a < 3; a++) rw += std::fabs(c[a] - (double)cf[a]);
+        hsb[(size_t)i] = make_float4(cf[0], cf[1], cf[2], std::nextafter((float)rw, INFINITY));
     }
     for (int i = 0; i < s->num_materials; i++) {
         const rt_material& m = s->materials[i];

@@ -327,17 +327,27 @@ __device__ __forceinline__ bool test_face(const DScene& S, int gi, int gface, in
     return false;
 }
 
-// FP32 pre-test against the sphere's world-space BOUNDING sphere (centre, radius >= the
-// ellipsoid's largest semi-axis, both rounded outward at upload).  It may only say "missed"
-// when the exact test would: the margins are ~250x the FP32 rounding of the expression
-// (relative 1e-4 on |c-o|^2, 1e-3 on the radius).  Skips about half of the exact tests
-// (a sphere fills 52 % of its box' projected area).
+// FP32 pre-test against the sphere's world-space BOUNDING sphere.  It may only say "missed"
+// when the exact test would.  Skips about half of the exact tests (a sphere fills 52 % of its
+// box' projected area).  Error bound, with d a unit vector:
+//  * bs.xyz is the centre rounded to nearest FP32; bs.w >= the ellipsoid's largest semi-axis
+//    plus |c - bs.xyz|, rounded up (rt_api.cu), so the ball (bs.xyz, bs.w) holds the ellipsoid.
+//  * (float)o is within 2^-24 |o_i| of o per axis, i.e. within sqrt(3) 2^-24 |o|inf < 2^-23 |o|inf
+//    in distance.  A ray from (float)o parallel to the true ray passes within that distance of
+//    every point of the true ray, so growing the radius by 2^-23 |o|inf covers it.  Both terms
+//    are absolute: they grow with the coordinates, not with the sphere or |c - o|.
+//  * What is left is the rounding of the FP32 expressions below and of d: a few 2^-24
+//    relative to |c - o|^2 and to r.  The margins are far larger (1e-4 on |c - o|^2 and 1e-3
+//    on the radius).
+// The test is conservative at any |coordinate| where |c - o|^2 stays finite in FP32 (below
+// ~1e19); past that c2 is inf and the comparisons are false, so nothing is culled.
 __device__ __forceinline__ bool sphere_certainly_missed(float4 bs, d3 o, d3 d) {
-    float ocx = bs.x - (float)o.x, ocy = bs.y - (float)o.y, ocz = bs.z - (float)o.z;
+    const float ox = (float)o.x, oy = (float)o.y, oz = (float)o.z;
+    float ocx = bs.x - ox, ocy = bs.y - oy, ocz = bs.z - oz;
     float dx = (float)d.x, dy = (float)d.y, dz = (float)d.z;
     float c2 = ocx * ocx + ocy * ocy + ocz * ocz;
     float b = ocx * dx + ocy * dy + ocz * dz;
-    float r = bs.w * 1.001f;
+    float r = (bs.w + 0x1p-23f * fmaxf(fabsf(ox), fmaxf(fabsf(oy), fabsf(oz)))) * 1.001f;
     float r2 = r * r + 1e-4f * c2 + 1e-30f;
     if (c2 - b * b > r2) return true;                       // the line passes outside the sphere
     return c2 > r2 && b < -(r + 1e-3f * sqrtf(c2));        // origin outside and the sphere entirely behind it
@@ -377,14 +387,21 @@ struct FRay {
     // direction component is >= 0, upper plane otherwise); the far plane is at address ^ 64
     unsigned nx, ny, nz;
 };
+// A direction component below `tiny` is clamped to +-tiny.  tiny >= |o_axis| 2^-126 keeps
+// |b| = |o| / tiny <= 2^126, finite: with a fixed 1e-30 an axis-parallel ray from |o| > 3.4e8
+// got b = +-inf, both plane distances of that axis +-inf, and missed every box.  The clamp
+// tilts the ray by at most tiny per unit of distance.  A hit lies within 3.5 M of the origin
+// (M: the padding's scale, see slab1), so the tilt stays <= 3.5 M max(1e-30, M 2^-126), below
+// the padding's 1e-6 M slack for M < 2e31.
 __device__ __forceinline__ FRay make_fray(d3 o, d3 d) {
     FRay r;
     float ox = (float)o.x, oy = (float)o.y, oz = (float)o.z;
     float dx = (float)d.x, dy = (float)d.y, dz = (float)d.z;
-    const float tiny = 1e-30f;
-    if (fabsf(dx) < tiny) dx = copysignf(tiny, dx);
-    if (fabsf(dy) < tiny) dy = copysignf(tiny, dy);
-    if (fabsf(dz) < tiny) dz = copysignf(tiny, dz);
+    const float tx = fmaxf(1e-30f, fabsf(ox) * 0x1p-126f), ty = fmaxf(1e-30f, fabsf(oy) * 0x1p-126f),
+                tz = fmaxf(1e-30f, fabsf(oz) * 0x1p-126f);
+    if (fabsf(dx) < tx) dx = copysignf(tx, dx);
+    if (fabsf(dy) < ty) dy = copysignf(ty, dy);
+    if (fabsf(dz) < tz) dz = copysignf(tz, dz);
     r.ix = 1.0f / dx; r.iy = 1.0f / dy; r.iz = 1.0f / dz;
     r.bx = -ox * r.ix; r.by = -oy * r.iy; r.bz = -oz * r.iz;
     r.nx = r.ix < 0.f ? 64u : 0u;
