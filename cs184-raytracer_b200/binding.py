@@ -92,6 +92,7 @@ RT_SYMBOLS = [
     "rt_unpack_tiles_rgb8", "rt_unpack_tiles", "rt_primary_ids", "rt_cast_rays", "rt_get_stats",
     "rt_microbench_gather", "rt_scene_device_bytes", "rt_intersection_max", "rt_divide_device",
     "rt_shared_frame_create", "rt_shared_frame_open", "rt_shared_frame_close", "rt_microbench_node_walk",
+    "rt_scene_refit",
 ]
 
 _rt = None
@@ -118,6 +119,7 @@ def load_rt() -> C.CDLL:
         lib.rt_create.argtypes = [C.c_int, C.POINTER(C.c_void_p)]
         lib.rt_destroy.argtypes = [C.c_void_p]
         lib.rt_scene_upload.argtypes = [C.c_void_p, C.c_void_p]
+        lib.rt_scene_refit.argtypes = [C.c_void_p, C.c_void_p]
         lib.rt_render.argtypes = [C.c_void_p, C.POINTER(rt_params), C.c_void_p, C.c_void_p, C.c_void_p]
         lib.rt_render_rgb8.argtypes = [C.c_void_p, C.POINTER(rt_params), C.c_void_p, C.c_void_p, C.c_void_p]
         lib.rt_render_device.argtypes = [C.c_void_p, C.POINTER(rt_params), C.c_void_p, C.c_void_p]
@@ -280,6 +282,13 @@ class Renderer:
         flat = scene.flat if isinstance(scene, HostScene) else scene
         self._scene_keepalive = scene
         self._check(self.lib.rt_scene_upload(self._h, C.cast(flat, C.c_void_p)), "rt_scene_upload")
+
+    def refit(self, scene):
+        """Update the uploaded scene to `scene` (HostScene or flat descriptor of the same structure) and refit the
+        LBVH instead of rebuilding it (rt_scene_refit)."""
+        flat = scene.flat if isinstance(scene, HostScene) else scene
+        self._check(self.lib.rt_scene_refit(self._h, C.cast(flat, C.c_void_p)), "rt_scene_refit")
+        self._scene_keepalive = scene
 
     def render(self, width, height, bounce_depth=10, intersection_only=False, flags=0, samples=0, n_gpus=0) -> np.ndarray:
         p = make_params(width, height, bounce_depth, intersection_only, flags=flags, samples=samples, n_gpus=n_gpus)

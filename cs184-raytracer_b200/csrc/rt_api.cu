@@ -135,6 +135,16 @@ struct rt_context {
     DevBuf<int> flat, all_prims, bvh_prims;
     DevBuf<float4> sph_bound;
     DevBuf<BvhNode> nodes;
+    DevBuf<int> node_level;                 // wide level of every node slot (build_lbvh), for the refit
+    size_t node_count = 0;
+    int bvh_levels = 0;
+    // Structure of the uploaded scene, which rt_scene_refit requires unchanged: (type, first_face, num_faces) per
+    // geometry, the face count and the FaceOwner table of k_pack_faces.  tri_pts: the six object-space points of
+    // every `tri` the device holds (a refit without faces derives the padding scale from them).
+    std::vector<int64_t> shape;
+    int64_t shape_faces = 0;
+    std::vector<FaceOwner> owners;
+    std::vector<double> tri_pts;
     DeviceArena scratch;                    // upload / LBVH-build temporaries
     // render state
     size_t cap = 0;                         // ray-queue capacity
@@ -288,13 +298,14 @@ void rt_destroy(rt_context* ctx) {
     delete ctx;
 }
 
-static int validate_scene(const rt_scene* s) {
+// faces_kept: a refit that keeps the faces on the device passes no face arrays.
+static int validate_scene(const rt_scene* s, bool faces_kept) {
     if (!s) return fail(RT_ERR_INVALID, "scene is NULL");
     if (s->num_geometries < 0 || s->num_lights < 0 || s->num_materials < 0 || s->num_faces < 0)
         return fail(RT_ERR_INVALID, "negative count in scene descriptor");
     if (s->num_faces > PRIM_INDEX_MASK) return fail(RT_ERR_INVALID, "too many faces (%lld)", (long long)s->num_faces);
     if ((s->num_geometries && !s->geometries) || (s->num_lights && !s->lights) ||
-        (s->num_materials && !s->materials) || (s->num_faces && (!s->face_points || !s->face_normals)))
+        (s->num_materials && !s->materials) || (s->num_faces && !faces_kept && (!s->face_points || !s->face_normals)))
         return fail(RT_ERR_INVALID, "NULL array in scene descriptor");
     for (int i = 0; i < s->num_geometries; i++) {
         const rt_geometry& g = s->geometries[i];
@@ -317,27 +328,35 @@ static int validate_scene(const rt_scene* s) {
     return RT_OK;
 }
 
-int rt_scene_upload(rt_context* ctx, const rt_scene* s) {
-    if (!ctx) return fail(RT_ERR_INVALID, "context is NULL");
-    int rc = validate_scene(s);
-    if (rc != RT_OK) return rc;
-    CU(cudaSetDevice(ctx->device));
-    ctx->have_scene = false;
-    ctx->sort_ok = false;
-    ctx->peers_stale = true;
-    cudaStream_t st = ctx->stream;
-    CU(cudaEventRecord(ctx->ev0, st));
-    int launches = 0;
-    const bool faces_on_device = (s->flags & RT_SCENE_FACES_ON_DEVICE) != 0;
+}  // extern "C"
 
-    // ---- host-side conversion of the small arrays ----
+namespace {
+
+// Host-side conversion of a scene descriptor, shared by rt_scene_upload and rt_scene_refit.
+struct SceneConv {
+    std::vector<DGeom> geoms;
+    std::vector<DMat> mats;
+    std::vector<DLight> slights, alights;
+    std::vector<float4> sph_bound;       // per geometry: world-space bounding sphere of a SPHERE (FP32 pre-test)
+    std::vector<int> simple_codes;       // prim codes of the spheres and `tri`s, geometry order
+    std::vector<double> simple_ext;      // world-space extent (largest axis) of each of them
+    double simple_lo[3] = {1e300, 1e300, 1e300}, simple_hi[3] = {-1e300, -1e300, -1e300};   // union of their boxes
+    std::vector<double> tri_pts;         // the six object-space points of every `tri`, geometry order
+    // Every point a ray of a render can start from is the camera eye or lies on a primitive: the largest
+    // |coordinate| of the eye and of the spheres and `tri`s (flat ones included; the LBVH primitives are measured
+    // on the device) scales the LBVH box padding, see slab1() in rt_device.cuh.
+    double origin_abs = 0;
+};
+
+// kept_tri_pts: the `tri` points to use when the descriptor carries no faces (a refit that keeps them), else null.
+int convert_scene(const rt_scene* s, const std::vector<double>* kept_tri_pts, SceneConv& c) {
     const int ng = s->num_geometries;
-    std::vector<DGeom> hg((size_t)ng);
-    std::vector<DMat> hm((size_t)s->num_materials);
-    std::vector<DLight> hsl, hal;
+    const bool faces_on_device = (s->flags & RT_SCENE_FACES_ON_DEVICE) != 0;
+    c.geoms.resize((size_t)ng);
+    c.mats.resize((size_t)s->num_materials);
     for (int i = 0; i < ng; i++) {
         const rt_geometry& g = s->geometries[i];
-        DGeom& d = hg[(size_t)i];
+        DGeom& d = c.geoms[(size_t)i];
         memset(&d, 0, sizeof(d));
         memcpy(d.inv, g.inv, sizeof(d.inv));
         memcpy(d.fwd, g.fwd, sizeof(d.fwd));
@@ -353,13 +372,13 @@ int rt_scene_upload(rt_context* ctx, const rt_scene* s) {
         d.use_bbox = g.use_bbox;
     }
     // world-space bounding spheres of the SPHERE geometries (FP32 pre-test, rt_device.cuh)
-    std::vector<float4> hsb((size_t)ng, make_float4(0.f, 0.f, 0.f, 0.f));
+    c.sph_bound.assign((size_t)ng, make_float4(0.f, 0.f, 0.f, 0.f));
     for (int i = 0; i < ng; i++) {
         const rt_geometry& g = s->geometries[i];
         if (g.type != RT_GEOM_SPHERE) continue;
-        double c[3], B[3][3] = {{0, 0, 0}, {0, 0, 0}, {0, 0, 0}};     // B = A^T A, A = linear part of fwd
+        double cw[3], B[3][3] = {{0, 0, 0}, {0, 0, 0}, {0, 0, 0}};     // B = A^T A, A = linear part of fwd
         for (int a = 0; a < 3; a++) {
-            c[a] = g.fwd[4 * a] * g.center[0] + g.fwd[4 * a + 1] * g.center[1] + g.fwd[4 * a + 2] * g.center[2] + g.fwd[4 * a + 3];
+            cw[a] = g.fwd[4 * a] * g.center[0] + g.fwd[4 * a + 1] * g.center[1] + g.fwd[4 * a + 2] * g.center[2] + g.fwd[4 * a + 3];
             for (int i2 = 0; i2 < 3; i2++)
                 for (int j2 = 0; j2 < 3; j2++) B[i2][j2] += g.fwd[4 * a + i2] * g.fwd[4 * a + j2];
         }
@@ -381,14 +400,14 @@ int rt_scene_upload(rt_context* ctx, const rt_scene* s) {
             lmax = q + 2 * p * std::cos(std::acos(r) / 3);
         }
         // the stored centre is c rounded to FP32: grow the radius by that rounding (sum of the axes >= its length)
-        const float cf[3] = {(float)c[0], (float)c[1], (float)c[2]};
+        const float cf[3] = {(float)cw[0], (float)cw[1], (float)cw[2]};
         double rw = std::fabs(g.radius) * std::sqrt(std::fmax(lmax, 0.0)) * (1.0 + 1e-6);
-        for (int a = 0; a < 3; a++) rw += std::fabs(c[a] - (double)cf[a]);
-        hsb[(size_t)i] = make_float4(cf[0], cf[1], cf[2], std::nextafter((float)rw, INFINITY));
+        for (int a = 0; a < 3; a++) rw += std::fabs(cw[a] - (double)cf[a]);
+        c.sph_bound[(size_t)i] = make_float4(cf[0], cf[1], cf[2], std::nextafter((float)rw, INFINITY));
     }
     for (int i = 0; i < s->num_materials; i++) {
         const rt_material& m = s->materials[i];
-        DMat& d = hm[(size_t)i];
+        DMat& d = c.mats[(size_t)i];
         memset(&d, 0, sizeof(d));
         memcpy(d.ka, m.ka, sizeof(d.ka));
         memcpy(d.kd, m.kd, sizeof(d.kd));
@@ -407,20 +426,168 @@ int rt_scene_upload(rt_context* ctx, const rt_scene* s) {
         memcpy(d.color, l.color, sizeof(d.color));
         d.falloff = l.falloff;
         d.type = l.type;
-        (l.type == RT_LIGHT_AMBIENT ? hal : hsl).push_back(d);
+        (l.type == RT_LIGHT_AMBIENT ? c.alights : c.slights).push_back(d);
     }
+    // world-space extent of every sphere / `tri` (few: host side)
+    for (int i = 0; i < ng; i++) {
+        const rt_geometry& g = s->geometries[i];
+        if (g.type == RT_GEOM_SPHERE || g.type == RT_GEOM_TRI)
+            c.simple_codes.push_back(((g.type == RT_GEOM_SPHERE ? PRIM_SPHERE : PRIM_TRI) << PRIM_KIND_SHIFT) | i);
+        if (g.type != RT_GEOM_TRI) continue;
+        if (kept_tri_pts) continue;
+        double six[18];
+        if (faces_on_device) CU(cudaMemcpy(six, s->face_points + 9 * g.first_face, sizeof(six), cudaMemcpyDeviceToHost));
+        else memcpy(six, s->face_points + 9 * g.first_face, sizeof(six));
+        c.tri_pts.insert(c.tri_pts.end(), six, six + 18);
+    }
+    if (kept_tri_pts) c.tri_pts = *kept_tri_pts;
+    c.simple_ext.assign(c.simple_codes.size(), 0.0);
+    for (int k = 0; k < 3; k++) c.origin_abs = std::fmax(c.origin_abs, std::fabs(s->camera.eye[k]));
+    size_t tri = 0;
+    for (size_t k = 0; k < c.simple_codes.size(); k++) {
+        const rt_geometry& g = s->geometries[c.simple_codes[k] & PRIM_INDEX_MASK];
+        double lo[3] = {1e300, 1e300, 1e300}, hi[3] = {-1e300, -1e300, -1e300};
+        auto grow = [&](const double* p) {
+            for (int a = 0; a < 3; a++) {
+                double w = g.fwd[4 * a] * p[0] + g.fwd[4 * a + 1] * p[1] + g.fwd[4 * a + 2] * p[2] + g.fwd[4 * a + 3];
+                lo[a] = std::fmin(lo[a], w);
+                hi[a] = std::fmax(hi[a], w);
+            }
+        };
+        if (g.type == RT_GEOM_SPHERE) {
+            for (int v = 0; v < 8; v++) {
+                double p[3] = {g.center[0] + ((v & 1) ? g.radius : -g.radius),
+                               g.center[1] + ((v & 2) ? g.radius : -g.radius),
+                               g.center[2] + ((v & 4) ? g.radius : -g.radius)};
+                grow(p);
+            }
+        } else {
+            for (int v = 0; v < 6; v++) grow(c.tri_pts.data() + 18 * tri + 3 * v);
+            tri++;
+        }
+        for (int a = 0; a < 3; a++) {
+            c.simple_ext[k] = std::fmax(c.simple_ext[k], hi[a] - lo[a]);
+            c.origin_abs = std::fmax(c.origin_abs, std::fmax(std::fabs(lo[a]), std::fabs(hi[a])));
+            c.simple_lo[a] = std::fmin(c.simple_lo[a], lo[a]);
+            c.simple_hi[a] = std::fmax(c.simple_hi[a], hi[a]);
+        }
+    }
+    return RT_OK;
+}
+
+// Arena bytes of an upload: the raw-face staging, then (reused) the LBVH build.  A refit of the same structure
+// reserves the same amount, so it never reallocates.
+size_t scene_scratch_bytes(const rt_scene* s, size_t n_owners, size_t n_simple, size_t n_bvh) {
+    const size_t nf = (size_t)s->num_faces;
+    const size_t need_faces = 2 * DeviceArena::padded(72 * nf) + DeviceArena::padded(sizeof(FaceOwner) * n_owners) +
+                              2 * DeviceArena::padded(4 * n_simple) + 4096;
+    return std::max(need_faces, lbvh_scratch_bytes(n_bvh));
+}
+
+// Raw faces (host or device memory, see RT_SCENE_FACES_ON_DEVICE) -> the 80-byte face records and the FACE codes
+// of all_prims / bvh_prims (k_pack_faces).  Host faces are staged in ctx->scratch.
+int pack_faces(rt_context* ctx, const rt_scene* s, const std::vector<FaceOwner>& owners, int* launches) {
+    cudaStream_t st = ctx->stream;
+    const size_t nf = (size_t)s->num_faces;
+    const double *raw_p = s->face_points, *raw_n = s->face_normals;
+    if (!(s->flags & RT_SCENE_FACES_ON_DEVICE)) {
+        double* up = ctx->scratch.take<double>(nf * 9);
+        double* un = ctx->scratch.take<double>(nf * 9);
+        if (!up || !un) return fail(RT_ERR_OOM, "upload scratch arena exhausted");
+        CU(cudaMemcpyAsync(up, s->face_points, sizeof(double) * 9 * nf, cudaMemcpyHostToDevice, st));
+        CU(cudaMemcpyAsync(un, s->face_normals, sizeof(double) * 9 * nf, cudaMemcpyHostToDevice, st));
+        raw_p = up; raw_n = un;
+    }
+    FaceOwner* d_owners = ctx->scratch.take<FaceOwner>(owners.size() ? owners.size() : 1);
+    if (!d_owners) return fail(RT_ERR_OOM, "upload scratch arena exhausted");
+    if (!owners.empty())
+        CU(cudaMemcpyAsync(d_owners, owners.data(), sizeof(FaceOwner) * owners.size(), cudaMemcpyHostToDevice, st));
+    k_pack_faces<<<(unsigned)((nf + 255) / 256), 256, 0, st>>>((long long)nf, raw_p, raw_n, d_owners, (int)owners.size(),
+                                                              ctx->face_pts.p, ctx->face_nrm.p, ctx->all_prims.p,
+                                                              ctx->bvh_prims.p);
+    (*launches)++;
+    LAUNCHED("k_pack_faces", st);
+    return RT_OK;
+}
+
+// The geometry, material and light tables to the device, and the DScene fields that point at them or count them
+// (the material and light counts may change between a scene and its refit).
+int upload_tables(rt_context* ctx, const rt_scene* s, const SceneConv& c) {
+    cudaStream_t st = ctx->stream;
+    CU(ctx->geoms.ensure(c.geoms.size()));
+    CU(ctx->sph_bound.ensure(c.geoms.size()));
+    CU(ctx->mats.ensure(c.mats.size()));
+    CU(ctx->slights.ensure(c.slights.size()));
+    CU(ctx->alights.ensure(c.alights.size()));
+    if (!c.geoms.empty()) {
+        CU(cudaMemcpyAsync(ctx->geoms.p, c.geoms.data(), sizeof(DGeom) * c.geoms.size(), cudaMemcpyHostToDevice, st));
+        CU(cudaMemcpyAsync(ctx->sph_bound.p, c.sph_bound.data(), sizeof(float4) * c.sph_bound.size(), cudaMemcpyHostToDevice, st));
+    }
+    if (!c.mats.empty()) CU(cudaMemcpyAsync(ctx->mats.p, c.mats.data(), sizeof(DMat) * c.mats.size(), cudaMemcpyHostToDevice, st));
+    if (!c.slights.empty()) CU(cudaMemcpyAsync(ctx->slights.p, c.slights.data(), sizeof(DLight) * c.slights.size(), cudaMemcpyHostToDevice, st));
+    if (!c.alights.empty()) CU(cudaMemcpyAsync(ctx->alights.p, c.alights.data(), sizeof(DLight) * c.alights.size(), cudaMemcpyHostToDevice, st));
+    DScene& S = ctx->S;
+    memcpy(&S.cam, &s->camera, sizeof(DCamera));
+    S.geoms = ctx->geoms.p;
+    S.sph_bound = ctx->sph_bound.p;
+    S.mats = ctx->mats.p;
+    S.slights = ctx->slights.p;
+    S.alights = ctx->alights.p;
+    S.num_geoms = (int)c.geoms.size();
+    S.num_slights = (int)c.slights.size();
+    S.num_alights = (int)c.alights.size();
+    ctx->used_geoms = c.geoms.size(); ctx->used_mats = c.mats.size();
+    ctx->used_slights = c.slights.size(); ctx->used_alights = c.alights.size();
+    return RT_OK;
+}
+
+// Bytes upload_tables copies.
+size_t table_bytes(const SceneConv& c) {
+    return sizeof(DGeom) * c.geoms.size() + sizeof(DMat) * c.mats.size() + sizeof(DLight) * (c.slights.size() + c.alights.size());
+}
+
+// Morton grid of the hit sort over the LBVH primitives' centroid bounds cb (min xyz, max xyz).
+void set_sort_grid(rt_context* ctx, const float* cb) {
+    float ext = 0.f;
+    for (int a = 0; a < 3; a++) ext = fmaxf(ext, cb[3 + a] - cb[a]);
+    ctx->sort_ok = ext > 0.f && std::isfinite(ext);
+    for (int a = 0; a < 3; a++) ctx->sort_grid.lo[a] = cb[a];
+    ctx->sort_grid.scale = ctx->sort_ok ? 1024.f / ext : 0.f;
+}
+
+}  // namespace
+
+extern "C" {
+
+int rt_scene_upload(rt_context* ctx, const rt_scene* s) {
+    if (!ctx) return fail(RT_ERR_INVALID, "context is NULL");
+    int rc = validate_scene(s, false);
+    if (rc != RT_OK) return rc;
+    CU(cudaSetDevice(ctx->device));
+    ctx->have_scene = false;
+    ctx->sort_ok = false;
+    ctx->peers_stale = true;
+    cudaStream_t st = ctx->stream;
+    CU(cudaEventRecord(ctx->ev0, st));
+    int launches = 0;
+    const bool faces_on_device = (s->flags & RT_SCENE_FACES_ON_DEVICE) != 0;
+
+    // ---- host-side conversion of the small arrays ----
+    const int ng = s->num_geometries;
+    SceneConv c;
+    if ((rc = convert_scene(s, nullptr, c)) != RT_OK) return rc;
+    const std::vector<int>& simple_codes = c.simple_codes;
 
     // ---- primitive codes: reference order, then the flat / BVH split ----
     // Only the per-GEOMETRY bookkeeping is done here; the per-face arrays (geometry / local
     // index of a face, FACE codes in reference and LBVH order) are expanded on the device by
     // k_pack_faces from the FaceOwner table.
-    std::vector<int> simple_codes, simple_all_pos;
+    std::vector<int> simple_all_pos;
     std::vector<FaceOwner> owners;
     size_t n_all = 0, n_mesh_faces = 0;
     for (int i = 0; i < ng; i++) {
         const rt_geometry& g = s->geometries[i];
         if (g.type == RT_GEOM_SPHERE || g.type == RT_GEOM_TRI) {
-            simple_codes.push_back(((g.type == RT_GEOM_SPHERE ? PRIM_SPHERE : PRIM_TRI) << PRIM_KIND_SHIFT) | i);
             simple_all_pos.push_back((int)n_all);
             n_all++;
         }
@@ -448,56 +615,16 @@ int rt_scene_upload(rt_context* ctx, const rt_scene* s) {
     // LBVH, except giants (floors) that would bloat its upper levels.
     std::vector<int> flat_codes, bvh_codes;
     const size_t kFlatMax = 64, kGiantMax = 16;
-    // world-space extent of every sphere / `tri` (few: host side)
-    std::vector<double> ext(simple_codes.size(), 0.0), pabs(simple_codes.size(), 0.0);
-    double ulo[3] = {1e300, 1e300, 1e300}, uhi[3] = {-1e300, -1e300, -1e300};
-    for (size_t k = 0; k < simple_codes.size(); k++) {
-        int code = simple_codes[k], gi = code & PRIM_INDEX_MASK;
-        const rt_geometry& g = s->geometries[gi];
-        double lo[3] = {1e300, 1e300, 1e300}, hi[3] = {-1e300, -1e300, -1e300};
-        auto grow = [&](const double* p) {
-            for (int a = 0; a < 3; a++) {
-                double w = g.fwd[4 * a] * p[0] + g.fwd[4 * a + 1] * p[1] + g.fwd[4 * a + 2] * p[2] + g.fwd[4 * a + 3];
-                lo[a] = std::fmin(lo[a], w);
-                hi[a] = std::fmax(hi[a], w);
-            }
-        };
-        if (g.type == RT_GEOM_SPHERE) {
-            for (int c = 0; c < 8; c++) {
-                double p[3] = {g.center[0] + ((c & 1) ? g.radius : -g.radius),
-                               g.center[1] + ((c & 2) ? g.radius : -g.radius),
-                               g.center[2] + ((c & 4) ? g.radius : -g.radius)};
-                grow(p);
-            }
-        } else {
-            double six[18];
-            if (faces_on_device) CU(cudaMemcpy(six, s->face_points + 9 * g.first_face, sizeof(six), cudaMemcpyDeviceToHost));
-            else memcpy(six, s->face_points + 9 * g.first_face, sizeof(six));
-            for (int v = 0; v < 6; v++) grow(six + 3 * v);
-        }
-        for (int a = 0; a < 3; a++) {
-            ext[k] = std::fmax(ext[k], hi[a] - lo[a]);
-            pabs[k] = std::fmax(pabs[k], std::fmax(std::fabs(lo[a]), std::fabs(hi[a])));
-            ulo[a] = std::fmin(ulo[a], lo[a]);
-            uhi[a] = std::fmax(uhi[a], hi[a]);
-        }
-    }
     if (simple_codes.size() <= kFlatMax) {
         flat_codes = simple_codes;
     } else {
         double uext = 0;
-        for (int a = 0; a < 3; a++) uext = std::fmax(uext, uhi[a] - ulo[a]);
+        for (int a = 0; a < 3; a++) uext = std::fmax(uext, c.simple_hi[a] - c.simple_lo[a]);
         for (size_t k = 0; k < simple_codes.size(); k++) {
-            if (ext[k] > 0.5 * uext && flat_codes.size() < kGiantMax) flat_codes.push_back(simple_codes[k]);
+            if (c.simple_ext[k] > 0.5 * uext && flat_codes.size() < kGiantMax) flat_codes.push_back(simple_codes[k]);
             else bvh_codes.push_back(simple_codes[k]);
         }
     }
-    // Every point a ray of a render can start from is the camera eye or lies on a primitive: the largest
-    // |coordinate| of the eye and of the primitives OUTSIDE the LBVH (those inside are measured on the device)
-    // scales the LBVH box padding, see slab1() in rt_device.cuh.
-    double origin_abs = 0;
-    for (int k = 0; k < 3; k++) origin_abs = std::fmax(origin_abs, std::fabs(s->camera.eye[k]));
-    for (size_t k = 0; k < simple_codes.size(); k++) origin_abs = std::fmax(origin_abs, pabs[k]);
     const int n_simple_in_bvh = (int)bvh_codes.size();       // bvh_codes: the simple part only (host copy)
     const size_t n_bvh = (size_t)n_simple_in_bvh + n_mesh_faces;
     for (FaceOwner& o : owners)
@@ -507,30 +634,18 @@ int rt_scene_upload(rt_context* ctx, const rt_scene* s) {
     const int group_first_code[2] = {n_simple_in_bvh ? bvh_codes[0] : 0, first_mesh_face_code};
 
     // ---- uploads ----
-    CU(ctx->geoms.ensure((size_t)ng));
-    CU(ctx->mats.ensure(hm.size()));
-    CU(ctx->slights.ensure(hsl.size()));
-    CU(ctx->alights.ensure(hal.size()));
-    CU(ctx->sph_bound.ensure((size_t)ng));
-    if (ng) CU(cudaMemcpyAsync(ctx->sph_bound.p, hsb.data(), sizeof(float4) * hsb.size(), cudaMemcpyHostToDevice, st));
+    DScene& S = ctx->S;
+    memset(&S, 0, sizeof(S));
+    if ((rc = upload_tables(ctx, s, c)) != RT_OK) return rc;
     CU(ctx->flat.ensure(flat_codes.size()));
     CU(ctx->all_prims.ensure(n_all));
     CU(ctx->bvh_prims.ensure(n_bvh));
     CU(ctx->face_pts.ensure((size_t)s->num_faces * RT_FACE_D2));
     CU(ctx->face_nrm.ensure((size_t)s->num_faces * RT_FACE_D2));
-    if (ng) CU(cudaMemcpyAsync(ctx->geoms.p, hg.data(), sizeof(DGeom) * hg.size(), cudaMemcpyHostToDevice, st));
-    if (!hm.empty()) CU(cudaMemcpyAsync(ctx->mats.p, hm.data(), sizeof(DMat) * hm.size(), cudaMemcpyHostToDevice, st));
-    if (!hsl.empty()) CU(cudaMemcpyAsync(ctx->slights.p, hsl.data(), sizeof(DLight) * hsl.size(), cudaMemcpyHostToDevice, st));
-    if (!hal.empty()) CU(cudaMemcpyAsync(ctx->alights.p, hal.data(), sizeof(DLight) * hal.size(), cudaMemcpyHostToDevice, st));
     if (!flat_codes.empty()) CU(cudaMemcpyAsync(ctx->flat.p, flat_codes.data(), sizeof(int) * flat_codes.size(), cudaMemcpyHostToDevice, st));
     if (!bvh_codes.empty()) CU(cudaMemcpyAsync(ctx->bvh_prims.p, bvh_codes.data(), sizeof(int) * bvh_codes.size(), cudaMemcpyHostToDevice, st));
-    {   // one arena reservation covers the raw-face staging and (afterwards, reused) the LBVH build
-        const size_t nf = (size_t)s->num_faces;
-        size_t need_faces = 2 * DeviceArena::padded(72 * nf) + DeviceArena::padded(sizeof(FaceOwner) * owners.size()) +
-                            2 * DeviceArena::padded(4 * simple_codes.size()) + 4096;
-        size_t need_build = lbvh_scratch_bytes(n_bvh);
-        CU(ctx->scratch.reserve(std::max(need_faces, need_build)));
-    }
+    // one arena reservation covers the raw-face staging and (afterwards, reused) the LBVH build
+    CU(ctx->scratch.reserve(scene_scratch_bytes(s, owners.size(), simple_codes.size(), n_bvh)));
     if (!simple_codes.empty()) {
         int* d_pos = ctx->scratch.take<int>(simple_codes.size());
         int* d_code = ctx->scratch.take<int>(simple_codes.size());
@@ -542,45 +657,14 @@ int rt_scene_upload(rt_context* ctx, const rt_scene* s) {
         launches++;
         LAUNCHED("k_scatter_codes", st);
     }
-    if (s->num_faces) {
-        const size_t nf = (size_t)s->num_faces;
-        const double *raw_p = s->face_points, *raw_n = s->face_normals;
-        if (!faces_on_device) {
-            double* up = ctx->scratch.take<double>(nf * 9);
-            double* un = ctx->scratch.take<double>(nf * 9);
-            if (!up || !un) return fail(RT_ERR_OOM, "upload scratch arena exhausted");
-            CU(cudaMemcpyAsync(up, s->face_points, sizeof(double) * 9 * nf, cudaMemcpyHostToDevice, st));
-            CU(cudaMemcpyAsync(un, s->face_normals, sizeof(double) * 9 * nf, cudaMemcpyHostToDevice, st));
-            raw_p = up; raw_n = un;
-        }
-        FaceOwner* d_owners = ctx->scratch.take<FaceOwner>(owners.size() ? owners.size() : 1);
-        if (!d_owners) return fail(RT_ERR_OOM, "upload scratch arena exhausted");
-        if (!owners.empty())
-            CU(cudaMemcpyAsync(d_owners, owners.data(), sizeof(FaceOwner) * owners.size(), cudaMemcpyHostToDevice, st));
-        k_pack_faces<<<(unsigned)((nf + 255) / 256), 256, 0, st>>>((long long)nf, raw_p, raw_n, d_owners, (int)owners.size(),
-                                                                  ctx->face_pts.p, ctx->face_nrm.p, ctx->all_prims.p,
-                                                                  ctx->bvh_prims.p);
-        launches++;
-        LAUNCHED("k_pack_faces", st);
-    }
+    if (s->num_faces && (rc = pack_faces(ctx, s, owners, &launches)) != RT_OK) return rc;
     CU(cudaStreamSynchronize(st));
     ctx->scratch.reset();
 
-    DScene& S = ctx->S;
-    memset(&S, 0, sizeof(S));
-    memcpy(&S.cam, &s->camera, sizeof(DCamera));
-    S.geoms = ctx->geoms.p;
-    S.mats = ctx->mats.p;
-    S.slights = ctx->slights.p;
-    S.alights = ctx->alights.p;
     S.face_pts = ctx->face_pts.p;
     S.face_nrm = ctx->face_nrm.p;
     S.flat = ctx->flat.p;
     S.all_prims = ctx->all_prims.p;
-    S.sph_bound = ctx->sph_bound.p;
-    S.num_geoms = ng;
-    S.num_slights = (int)hsl.size();
-    S.num_alights = (int)hal.size();
     S.num_flat = (int)flat_codes.size();
     S.num_all = (int)n_all;
     S.num_bvh_prims = (int)n_bvh;
@@ -590,23 +674,22 @@ int rt_scene_upload(rt_context* ctx, const rt_scene* s) {
     // ---- LBVH ----
     cudaEvent_t evb = ctx->ev_build;
     size_t node_count = 0;
+    int levels = 0;
     S.origin_limit = 3.0e38f;
     if (n_bvh >= 2) {
-        const float extra_abs = std::nextafter((float)origin_abs, INFINITY);
+        const float extra_abs = std::nextafter((float)c.origin_abs, INFINITY);
         char err[256] = "";
         float cb[6] = {0, 0, 0, 0, 0, 0};
         float pad_scale = 0.f;
         CU(ctx->nodes.ensure(n_bvh + 2));
+        CU(ctx->node_level.ensure(n_bvh + 2));
         int brc = build_lbvh(S, ctx->bvh_prims.p, group_first_code, (int)n_bvh, group_sizes, 2, extra_abs, st,
-                             ctx->scratch, ctx->nodes.p, &node_count, &launches, err, sizeof(err), cb, &pad_scale);
+                             ctx->scratch, ctx->nodes.p, &node_count, &launches, err, sizeof(err), cb, &pad_scale,
+                             ctx->node_level.p, &levels);
         ctx->scratch.reset();
         if (brc != RT_OK) return fail(brc, "LBVH build: %s", err);
         S.origin_limit = pad_scale;
-        float ext = 0.f;
-        for (int a = 0; a < 3; a++) ext = fmaxf(ext, cb[3 + a] - cb[a]);
-        ctx->sort_ok = ext > 0.f && std::isfinite(ext);
-        for (int a = 0; a < 3; a++) ctx->sort_grid.lo[a] = cb[a];
-        ctx->sort_grid.scale = ctx->sort_ok ? 1024.f / ext : 0.f;
+        set_sort_grid(ctx, cb);
     }
     S.nodes = node_count ? ctx->nodes.p : nullptr;
     cudaEventRecord(evb, st);
@@ -614,15 +697,93 @@ int rt_scene_upload(rt_context* ctx, const rt_scene* s) {
     float ms0 = 0, ms1 = 0;
     cudaEventElapsedTime(&ms0, ctx->ev0, ctx->ev1);
     cudaEventElapsedTime(&ms1, ctx->ev1, evb);
-    ctx->used_geoms = (size_t)ng; ctx->used_mats = hm.size(); ctx->used_slights = hsl.size(); ctx->used_alights = hal.size();
     ctx->used_faces = (size_t)s->num_faces; ctx->used_flat = flat_codes.size(); ctx->used_all = n_all;
     ctx->used_nodes = node_count ? n_bvh + 2 : 0;
+    ctx->node_count = node_count;
+    ctx->bvh_levels = levels;
     ctx->node_bytes = sizeof(BvhNode) * node_count;
     ctx->face_bytes = sizeof(double2) * RT_FACE_D2 * 2 * (size_t)s->num_faces;
-    ctx->stats.scene_bytes_h2d = sizeof(DGeom) * hg.size() + sizeof(DMat) * hm.size() +
-                                 sizeof(DLight) * (hsl.size() + hal.size()) +
-                                 sizeof(int) * (flat_codes.size() + 2 * simple_codes.size() + bvh_codes.size()) +
+    ctx->shape_faces = s->num_faces;
+    ctx->shape.resize(3 * (size_t)ng);
+    for (int i = 0; i < ng; i++) {
+        ctx->shape[3 * (size_t)i] = s->geometries[i].type;
+        ctx->shape[3 * (size_t)i + 1] = s->geometries[i].first_face;
+        ctx->shape[3 * (size_t)i + 2] = s->geometries[i].num_faces;
+    }
+    ctx->owners = owners;
+    ctx->tri_pts = std::move(c.tri_pts);
+    ctx->stats.scene_bytes_h2d = table_bytes(c) + sizeof(int) * (flat_codes.size() + 2 * simple_codes.size() + bvh_codes.size()) +
                                  sizeof(FaceOwner) * owners.size() + (faces_on_device ? 0 : (size_t)s->num_faces * (2 * 72));
+    ctx->stats.ms_upload = ms0;
+    ctx->stats.ms_build = ms1;
+    ctx->stats.kernel_launches = (uint64_t)launches;
+    ctx->have_scene = true;
+    return RT_OK;
+}
+
+int rt_scene_refit(rt_context* ctx, const rt_scene* s) {
+    // ---- validation: nothing is written before it passes ----
+    if (!ctx) return fail(RT_ERR_INVALID, "context is NULL");
+    if (!ctx->have_scene) return fail(RT_ERR_NO_SCENE, "rt_scene_refit: rt_scene_upload has not been called");
+    if (s && (s->face_points == nullptr) != (s->face_normals == nullptr))
+        return fail(RT_ERR_INVALID, "rt_scene_refit: face_points and face_normals must both be set or both be NULL");
+    const bool keep_faces = s && s->face_points == nullptr;
+    int rc = validate_scene(s, keep_faces);
+    if (rc != RT_OK) return rc;
+    const int ng = s->num_geometries;
+    if ((size_t)ng * 3 != ctx->shape.size())
+        return fail(RT_ERR_INVALID, "rt_scene_refit: num_geometries %d differs from the uploaded scene's %zu", ng,
+                    ctx->shape.size() / 3);
+    if (s->num_faces != ctx->shape_faces)
+        return fail(RT_ERR_INVALID, "rt_scene_refit: num_faces %lld differs from the uploaded scene's %lld",
+                    (long long)s->num_faces, (long long)ctx->shape_faces);
+    for (int i = 0; i < ng; i++) {
+        const rt_geometry& g = s->geometries[i];
+        const int64_t* u = ctx->shape.data() + 3 * (size_t)i;
+        const int64_t got[3] = {g.type, g.first_face, g.num_faces};
+        static const char* const field[3] = {"type", "first_face", "num_faces"};
+        for (int f = 0; f < 3; f++)
+            if (got[f] != u[f])
+                return fail(RT_ERR_INVALID, "rt_scene_refit: geometry %d: %s %lld differs from the uploaded scene's %lld", i,
+                            field[f], (long long)got[f], (long long)u[f]);
+    }
+    CU(cudaSetDevice(ctx->device));
+    SceneConv c;
+    if ((rc = convert_scene(s, keep_faces ? &ctx->tri_pts : nullptr, c)) != RT_OK) return rc;
+
+    // ---- writes: from here a failure leaves no scene, like a failed upload ----
+    ctx->have_scene = false;
+    ctx->peers_stale = true;
+    cudaStream_t st = ctx->stream;
+    CU(cudaEventRecord(ctx->ev0, st));
+    int launches = 0;
+    if ((rc = upload_tables(ctx, s, c)) != RT_OK) return rc;
+    DScene& S = ctx->S;
+    // the upload reserved this much already: no allocation
+    CU(ctx->scratch.reserve(scene_scratch_bytes(s, ctx->owners.size(), c.simple_codes.size(), (size_t)S.num_bvh_prims)));
+    if (!keep_faces && s->num_faces && (rc = pack_faces(ctx, s, ctx->owners, &launches)) != RT_OK) return rc;
+    ctx->scratch.reset();       // the refit's launches are stream-ordered after k_pack_faces: the staging is free
+    CU(cudaEventRecord(ctx->ev1, st));
+    if (S.nodes) {
+        const float extra_abs = std::nextafter((float)c.origin_abs, INFINITY);
+        char err[256] = "";
+        float cb[6], pad_scale = 0.f;
+        int brc = refit_lbvh(S, ctx->bvh_prims.p, S.num_bvh_prims, ctx->node_level.p, ctx->bvh_levels, ctx->node_count,
+                             extra_abs, st, ctx->scratch, ctx->nodes.p, &launches, err, sizeof(err), cb, &pad_scale);
+        ctx->scratch.reset();
+        if (brc != RT_OK) return fail(brc, "LBVH refit: %s", err);
+        S.origin_limit = pad_scale;
+        set_sort_grid(ctx, cb);
+    }
+    CU(cudaEventRecord(ctx->ev_build, st));
+    CU(cudaStreamSynchronize(st));
+    float ms0 = 0, ms1 = 0;
+    cudaEventElapsedTime(&ms0, ctx->ev0, ctx->ev1);
+    cudaEventElapsedTime(&ms1, ctx->ev1, ctx->ev_build);
+    if (!keep_faces) ctx->tri_pts = std::move(c.tri_pts);
+    ctx->stats.scene_bytes_h2d = table_bytes(c) + sizeof(float4) * c.sph_bound.size() +
+                                 (keep_faces ? 0 : sizeof(FaceOwner) * ctx->owners.size()) +
+                                 (keep_faces || (s->flags & RT_SCENE_FACES_ON_DEVICE) ? 0 : (size_t)s->num_faces * (2 * 72));
     ctx->stats.ms_upload = ms0;
     ctx->stats.ms_build = ms1;
     ctx->stats.kernel_launches = (uint64_t)launches;
@@ -1522,11 +1683,13 @@ int rt_cast_rays(rt_context* ctx, int64_t n, const double* org, const double* di
     const size_t N = (size_t)n;
     CU(d_org.ensure(3 * N)); CU(d_dir.ensure(3 * N)); CU(d_dist.ensure(N)); CU(d_point.ensure(3 * N)); CU(d_normal.ensure(3 * N));
     CU(d_geom.ensure(N)); CU(d_face.ensure(N));
-    CU(cudaMemcpy(d_org.p, org, sizeof(double) * 3 * N, cudaMemcpyHostToDevice));
-    CU(cudaMemcpy(d_dir.p, dir, sizeof(double) * 3 * N, cudaMemcpyHostToDevice));
+    // on the query's own stream: a cudaMemcpy from pageable memory may return before its DMA has landed, and the
+    // context's streams do not wait for the legacy default stream
+    CU(cudaMemcpyAsync(d_org.p, org, sizeof(double) * 3 * N, cudaMemcpyHostToDevice, ctx->stream));
+    CU(cudaMemcpyAsync(d_dir.p, dir, sizeof(double) * 3 * N, cudaMemcpyHostToDevice, ctx->stream));
     if (reverse) {
         CU(d_rev.ensure(N));
-        CU(cudaMemcpy(d_rev.p, reverse, N, cudaMemcpyHostToDevice));
+        CU(cudaMemcpyAsync(d_rev.p, reverse, N, cudaMemcpyHostToDevice, ctx->stream));
     }
     const unsigned blocks = (unsigned)((N + RT_BLOCK - 1) / RT_BLOCK);
     if (flags & RT_FLAG_BRUTE_FORCE)

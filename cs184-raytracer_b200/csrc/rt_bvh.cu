@@ -32,12 +32,9 @@ __host__ __device__ __forceinline__ float ord2f(int i) {
 #endif
 }
 
-// World-space bounds of one primitive (FP64 math, rounded outward to FP32).
-__global__ void k_prim_bounds(DScene S, const int* __restrict__ codes, int n, float* __restrict__ lo,
-                              float* __restrict__ hi, int* __restrict__ gbounds /*[7]: cmin xyz, cmax xyz, maxabs*/) {
-    int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    int code = codes[i];
+// World-space bounds of the primitive with code `code` (FP64 math, rounded outward to FP32).  The build and the
+// refit both call this, so a refit of unchanged primitives reproduces the build's boxes bit for bit.
+__device__ __forceinline__ void prim_bounds(const DScene& S, int code, float lo[3], float hi[3]) {
     int kind = code >> PRIM_KIND_SHIFT, idx = code & PRIM_INDEX_MASK;
     double mn[3] = {DBL_MAX, DBL_MAX, DBL_MAX}, mx[3] = {-DBL_MAX, -DBL_MAX, -DBL_MAX};
     auto grow = [&](d3 p) {
@@ -71,9 +68,21 @@ __global__ void k_prim_bounds(DScene S, const int* __restrict__ codes, int n, fl
         double2 q4 = S.face_pts[(size_t)idx * RT_FACE_D2 + 4];
         face_bounds(idx, S.geoms + __double2loint(q4.y));
     }
+    for (int a = 0; a < 3; a++) {
+        lo[a] = __double2float_rd(mn[a]);
+        hi[a] = __double2float_ru(mx[a]);
+    }
+}
+
+__global__ void k_prim_bounds(DScene S, const int* __restrict__ codes, int n, float* __restrict__ lo,
+                              float* __restrict__ hi, int* __restrict__ gbounds /*[7]: cmin xyz, cmax xyz, maxabs*/) {
+    int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    float pl[3], ph[3];
+    prim_bounds(S, codes[i], pl, ph);
     float maxabs = 0.f;
     for (int a = 0; a < 3; a++) {
-        float l = __double2float_rd(mn[a]), h = __double2float_ru(mx[a]);
+        float l = pl[a], h = ph[a];
         lo[3 * (size_t)i + a] = l;
         hi[3 * (size_t)i + a] = h;
         float c = 0.5f * l + 0.5f * h;
@@ -440,23 +449,32 @@ __global__ void k_choose_children(int n, int wave, int* __restrict__ wave_of, in
     slots4[i] = make_int4(slots[0], slots[1], slots[2], slots[3]);
 }
 
+// Padding of every stored child box: a few FP32 ulps at the scene's largest coordinate M (covers the slab test's
+// rounding), plus a relative margin.  The build and the refit share these, so equal boxes give equal bytes.
+__host__ __device__ __forceinline__ float box_pad(float m) { return 2e-6f * fmaxf(m, 1e-30f); }
+__host__ __device__ __forceinline__ float pad_lo(float l, float pad) { return l - pad - fabsf(l) * 2e-7f; }
+__host__ __device__ __forceinline__ float pad_hi(float h, float pad) { return h + pad + fabsf(h) * 2e-7f; }
+
 // Binary Karras nodes at EVEN depth become 4-wide nodes: each internal child (odd depth) is
 // replaced by its own two children.  Wide nodes keep the binary node's index (+ offset), so
 // no compaction pass is needed; odd-depth slots of the array stay unused.
 //
 // slots4 != null: the children were chosen by k_choose_children (wave_of[i] >= 0 marks the wide nodes) instead.
+// node_level[node_offset + i]: the wide level of slot i (+ level_base), -1 for a slot that holds no node; the
+// refit (k_refit_wide) visits the levels deepest first.
 __global__ void k_pack_wide(int n, const int* __restrict__ vals, const int* __restrict__ codes,
                             const float* __restrict__ plo, const float* __restrict__ phi,
                             const int* __restrict__ left, const int* __restrict__ right,
                             const float* __restrict__ ilo, const float* __restrict__ ihi,
                             const int* __restrict__ depth, const int* __restrict__ gbounds,
                             BvhNode* __restrict__ nodes, int node_offset, const int* __restrict__ wave_of,
-                            const int4* __restrict__ slots4) {
+                            const int4* __restrict__ slots4, int* __restrict__ node_level, int level_base) {
     int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n - 1) return;
-    if (slots4 ? wave_of[i] < 0 : (depth[i] & 1) != 0) return;
-    // pad: a few FP32 ulps at the scene's largest coordinate (covers the slab test's rounding)
-    const float pad = 2e-6f * fmaxf(ord2f(gbounds[6]), 1e-30f);
+    const int level = slots4 ? wave_of[i] : ((depth[i] & 1) ? -1 : depth[i] >> 1);
+    node_level[node_offset + i] = level < 0 ? -1 : level + level_base;
+    if (level < 0) return;
+    const float pad = box_pad(ord2f(gbounds[6]));
     int slots[4];
     int ns = 0;
     int ch[2] = {left[i], right[i]};
@@ -490,9 +508,8 @@ __global__ void k_pack_wide(int n, const int* __restrict__ vals, const int* __re
             ref[k] = slots[k] + node_offset;
         }
         for (int a = 0; a < 3; a++) {
-            float l = bl[a], h = bh[a];
-            lo[a][k] = l - pad - fabsf(l) * 2e-7f;
-            hi[a][k] = h + pad + fabsf(h) * 2e-7f;
+            lo[a][k] = pad_lo(bl[a], pad);
+            hi[a][k] = pad_hi(bh[a], pad);
         }
     }
     BvhNode nd;
@@ -505,6 +522,49 @@ __global__ void k_pack_wide(int n, const int* __restrict__ vals, const int* __re
     nd.ref = make_int4(ref[0], ref[1], ref[2], ref[3]);
     nd.pad_ = make_int4(0, 0, 0, 0);
     nodes[node_offset + i] = nd;
+}
+
+// Refit of the wide nodes of one level (node_level[i] == level), launched for the levels deepest first: every slot
+// gets a new box and keeps its reference.  A leaf slot takes its primitive's bounds; an internal slot takes the
+// unpadded union of its child's four slots (ubox, 6 floats per node, written by the launch of the level below),
+// which covers the same leaves as the build's binary box of that child and therefore equals it bit for bit.
+__global__ void k_refit_wide(DScene S, int count, int level, const int* __restrict__ node_level,
+                             const int* __restrict__ gbounds, BvhNode* __restrict__ nodes, float* __restrict__ ubox) {
+    int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= count || node_level[i] != level) return;
+    const float pad = box_pad(ord2f(gbounds[6]));
+    const int4 r4 = nodes[i].ref;
+    const int ref[4] = {r4.x, r4.y, r4.z, r4.w};
+    float lo[3][4], hi[3][4], u[6] = {FLT_MAX, FLT_MAX, FLT_MAX, -FLT_MAX, -FLT_MAX, -FLT_MAX};
+    for (int k = 0; k < 4; k++) {
+        if (ref[k] == BVH_DONE) {
+            for (int a = 0; a < 3; a++) { lo[a][k] = BVH_EMPTY_LO; hi[a][k] = BVH_EMPTY_HI; }
+            continue;
+        }
+        float bl[3], bh[3];
+        if (ref[k] < 0) {
+            prim_bounds(S, ~ref[k], bl, bh);
+        } else {
+            for (int a = 0; a < 3; a++) { bl[a] = ubox[6 * (size_t)ref[k] + a]; bh[a] = ubox[6 * (size_t)ref[k] + 3 + a]; }
+        }
+        for (int a = 0; a < 3; a++) {
+            u[a] = fminf(u[a], bl[a]);
+            u[3 + a] = fmaxf(u[3 + a], bh[a]);
+            lo[a][k] = pad_lo(bl[a], pad);
+            hi[a][k] = pad_hi(bh[a], pad);
+        }
+    }
+    for (int a = 0; a < 6; a++) ubox[6 * (size_t)i + a] = u[a];
+    BvhNode nd;
+    nd.lox = make_float4(lo[0][0], lo[0][1], lo[0][2], lo[0][3]);
+    nd.loy = make_float4(lo[1][0], lo[1][1], lo[1][2], lo[1][3]);
+    nd.loz = make_float4(lo[2][0], lo[2][1], lo[2][2], lo[2][3]);
+    nd.hix = make_float4(hi[0][0], hi[0][1], hi[0][2], hi[0][3]);
+    nd.hiy = make_float4(hi[1][0], hi[1][1], hi[1][2], hi[1][3]);
+    nd.hiz = make_float4(hi[2][0], hi[2][1], hi[2][2], hi[2][3]);
+    nd.ref = r4;
+    nd.pad_ = make_int4(0, 0, 0, 0);
+    nodes[i] = nd;
 }
 
 #define TAKE(var, type, count)                                                         \
@@ -530,8 +590,10 @@ __global__ void k_pack_wide(int n, const int* __restrict__ vals, const int* __re
 // otherwise stretch the leaf-level boxes of the mesh over the whole air space.
 int build_lbvh(const DScene& S, const int* d_codes, const int* group_first_code, int n, const int* group_sizes, int ngroups,
                float extra_abs, cudaStream_t stream, DeviceArena& arena, BvhNode* nodes, size_t* out_count,
-               int* launches, char* err, int errlen, float* centroid_bounds, float* out_pad_scale) {
+               int* launches, char* err, int errlen, float* centroid_bounds, float* out_pad_scale, int* node_level,
+               int* out_levels) {
     *out_count = 0;
+    *out_levels = 0;
     float *plo = nullptr, *phi = nullptr, *ilo = nullptr, *ihi = nullptr;
     int *gb = nullptr, *vals0 = nullptr, *vals1 = nullptr, *hist = nullptr;
     int4* slots4 = nullptr;
@@ -545,7 +607,7 @@ int build_lbvh(const DScene& S, const int* d_codes, const int* group_first_code,
     float pad_scale = 0.f;
     struct Group { int start, n, root_ref, first_code; float box[6]; };
     Group groups[4];
-    int K = 0;
+    int K = 0, levels = 0;
     size_t total_nodes = 0;
     {
         if (n < 2 || ngroups > 4) return RT_OK;    // nothing to build (caller tests a single primitive directly)
@@ -598,6 +660,7 @@ int build_lbvh(const DScene& S, const int* d_codes, const int* group_first_code,
         TAKE(wdepth, int, (size_t)n);
         k_morton<<<nblk, T, 0, stream>>>(plo, phi, n, gb, keys0, vals0);
         (*launches)++;
+        if (nsuper) CK(cudaMemsetAsync(node_level, 0, sizeof(int), stream));     // the super node: the last level refit
         size_t node_cursor = (size_t)nsuper;
         for (int g = 0; g < K; g++) {
             const int gs = groups[g].start, gn = groups[g].n;
@@ -654,8 +717,9 @@ int build_lbvh(const DScene& S, const int* d_codes, const int* group_first_code,
                         (*launches)++;
                     }
                     k_pack_wide<<<gblk, T, 0, stream>>>(gn, vin, d_codes, plo, phi, gleft, gright, gilo, gihi, nullptr, gb,
-                                                        nodes, (int)node_cursor, wave_of, slots4 + gs);
+                                                        nodes, (int)node_cursor, wave_of, slots4 + gs, node_level, nsuper);
                     (*launches)++;
+                    levels = std::max(levels, nsuper + wide_depth);
                     break;
                 }
                 CK(cudaMemsetAsync(gb + 7, 0, sizeof(int), stream));
@@ -671,8 +735,9 @@ int build_lbvh(const DScene& S, const int* d_codes, const int* group_first_code,
                     return RT_ERR_LIMIT;
                 }
                 k_pack_wide<<<gblk, T, 0, stream>>>(gn, vin, d_codes, plo, phi, gleft, gright, gilo, gihi, depth + gs, gb,
-                                                    nodes, (int)node_cursor, nullptr, nullptr);
+                                                    nodes, (int)node_cursor, nullptr, nullptr, node_level, nsuper);
                 (*launches)++;
+                levels = std::max(levels, nsuper + gdepth / 2 + 1);
             }
             groups[g].root_ref = (int)node_cursor;
             CK(cudaMemcpyAsync(groups[g].box, ilo + 3 * (size_t)gs, 12, cudaMemcpyDeviceToHost, stream));
@@ -681,8 +746,9 @@ int build_lbvh(const DScene& S, const int* d_codes, const int* group_first_code,
         }
         CK(cudaStreamSynchronize(stream));
         CK(cudaGetLastError());
+        levels = std::max(levels, nsuper);
         if (nsuper > 0) {
-            const float pad = 2e-6f * fmaxf(pad_scale, 1e-30f);
+            const float pad = box_pad(pad_scale);
             float lo[3][4], hi[3][4];
             int ref[4];
             for (int k = 0; k < 4; k++) {
@@ -691,9 +757,8 @@ int build_lbvh(const DScene& S, const int* d_codes, const int* group_first_code,
                 if (k >= K) continue;
                 ref[k] = groups[k].root_ref;
                 for (int a = 0; a < 3; a++) {
-                    float l = groups[k].box[a], h = groups[k].box[3 + a];
-                    lo[a][k] = l - pad - fabsf(l) * 2e-7f;
-                    hi[a][k] = h + pad + fabsf(h) * 2e-7f;
+                    lo[a][k] = pad_lo(groups[k].box[a], pad);
+                    hi[a][k] = pad_hi(groups[k].box[3 + a], pad);
                 }
             }
             BvhNode nd;
@@ -709,9 +774,50 @@ int build_lbvh(const DScene& S, const int* d_codes, const int* group_first_code,
         }
     }
     *out_count = total_nodes;
+    *out_levels = levels;
     if (out_pad_scale) *out_pad_scale = pad_scale;
     if (centroid_bounds)
         for (int a = 0; a < 6; a++) centroid_bounds[a] = ord2f(hb[a]);
+    return RT_OK;
+fail:
+    return RT_ERR_CUDA;
+}
+
+int refit_lbvh(const DScene& S, const int* d_codes, int n, const int* node_level, int levels, size_t node_count,
+               float extra_abs, cudaStream_t stream, DeviceArena& arena, BvhNode* nodes, int* launches, char* err,
+               int errlen, float* centroid_bounds, float* out_pad_scale) {
+    float *plo = nullptr, *phi = nullptr, *ubox = nullptr;
+    int* gb = nullptr;
+    const int T = 256;
+    int hb[7];
+    float m = 0.f;
+    {
+        TAKE(plo, float, 3 * (size_t)n);
+        TAKE(phi, float, 3 * (size_t)n);
+        TAKE(gb, int, 16);
+        TAKE(ubox, float, 6 * node_count);
+        const int init[7] = {0x7fffffff, 0x7fffffff, 0x7fffffff, (int)0x80000000, (int)0x80000000, (int)0x80000000,
+                             (int)0x80000000};
+        CK(cudaMemcpyAsync(gb, init, sizeof(init), cudaMemcpyHostToDevice, stream));
+        k_prim_bounds<<<(n + T - 1) / T, T, 0, stream>>>(S, d_codes, n, plo, phi, gb);
+        (*launches)++;
+        CK(cudaMemcpyAsync(hb, gb, sizeof(hb), cudaMemcpyDeviceToHost, stream));
+        CK(cudaStreamSynchronize(stream));
+        // M as build_lbvh derives it: the primitives' largest |coordinate| folded with extra_abs
+        m = ord2f(hb[6]);
+        if (extra_abs > m) m = extra_abs;
+        int enc;
+        memcpy(&enc, &m, 4);
+        CK(cudaMemcpyAsync(gb + 6, &enc, sizeof(int), cudaMemcpyHostToDevice, stream));
+        const unsigned blk = (unsigned)((node_count + T - 1) / T);
+        for (int l = levels - 1; l >= 0; l--) {
+            k_refit_wide<<<blk, T, 0, stream>>>(S, (int)node_count, l, node_level, gb, nodes, ubox);
+            (*launches)++;
+        }
+        CK(cudaGetLastError());
+    }
+    *out_pad_scale = m;
+    for (int a = 0; a < 6; a++) centroid_bounds[a] = ord2f(hb[a]);
     return RT_OK;
 fail:
     return RT_ERR_CUDA;

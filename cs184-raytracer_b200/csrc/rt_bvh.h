@@ -43,11 +43,24 @@ inline size_t lbvh_scratch_bytes(size_t n) {
 // joins them under super nodes so that node 0 is always the root, written to `nodes`
 // (caller-allocated).  n < 2 builds nothing (*out_count = 0).  Temporaries come from `arena`.  extra_abs: largest |coordinate| of ray origins outside the
 // primitives (the camera eye) and of the primitives kept OUT of the LBVH (flat list), folded into the box padding.
+// node_level (device, one int per node slot) receives the wide level of every node, root or super node = 0, and -1
+// for slots that hold no node; *out_levels the number of levels.  Both are what refit_lbvh needs.
 // Returns RT_OK, RT_ERR_CUDA or RT_ERR_LIMIT (too many nodes / tree deeper than the traversal stack).
 int build_lbvh(const DScene& S, const int* d_codes, const int* group_first_code, int n, const int* group_sizes, int ngroups,
                float extra_abs, cudaStream_t stream, DeviceArena& arena, BvhNode* nodes /* >= n + ngroups */,
                size_t* out_count, int* launches, char* err, int errlen,
                float* centroid_bounds /* [6] or null: min xyz, max xyz of the primitive centroids */,
-               float* out_pad_scale /* or null: the largest |coordinate| the box padding covers */);
+               float* out_pad_scale /* or null: the largest |coordinate| the box padding covers */,
+               int* node_level /* >= n + ngroups */, int* out_levels);
+
+// Recomputes every box of the node array build_lbvh wrote over the same n primitive codes, whose geometry (S) may
+// have changed, and keeps its topology: one bounds pass over d_codes (new M = largest |coordinate|, folded with
+// extra_abs as in the build, and the centroid bounds), then one launch per level, deepest first.  The padding is
+// the build's, so refitting unchanged primitives rewrites the node array byte for byte.  Takes 24 B per primitive and
+// per node from `arena`; synchronises `stream` once, after the bounds pass (M is needed on the host), and leaves the
+// level launches enqueued.  Returns RT_OK or RT_ERR_CUDA.
+int refit_lbvh(const DScene& S, const int* d_codes, int n, const int* node_level, int levels, size_t node_count,
+               float extra_abs, cudaStream_t stream, DeviceArena& arena, BvhNode* nodes, int* launches, char* err,
+               int errlen, float* centroid_bounds /* [6] */, float* out_pad_scale);
 
 }  // namespace rt

@@ -204,6 +204,33 @@ int  rt_abi_version(void);
  * (src/geometry.cpp:5-29) as the acceleration structure. */
 int  rt_scene_upload(rt_context* ctx, const rt_scene* scene);
 
+/* Update the uploaded scene in place and refit its LBVH instead of rebuilding it: for
+ * animation (a moving camera or light, rigid motion, deforming vertices) at a fraction of the
+ * cost of rt_scene_upload.
+ *   - The descriptor must have the STRUCTURE of the scene last uploaded to ctx: the same
+ *     num_geometries and num_faces, and per geometry the same type, first_face and num_faces.
+ *     Everything else may change: fwd, inv, det, center, radius, radius2, bbmin, bbmax,
+ *     use_bbox and material (range-checked); the materials and the lights, their counts
+ *     included; the camera; the face points and normals.
+ *   - face_points == NULL && face_normals == NULL: the faces on the device stay as they are.
+ *     Mesh faces are in object space, so a rigid motion changes only the transform and no face
+ *     bytes are copied.  Exactly one of the two NULL is RT_ERR_INVALID.  Otherwise the faces are
+ *     read as by rt_scene_upload, RT_SCENE_FACES_ON_DEVICE included.
+ *   - Errors: RT_ERR_NO_SCENE when nothing has been uploaded; RT_ERR_INVALID on a structure
+ *     mismatch (rt_last_error() names the first mismatching field and geometry index) or a
+ *     malformed descriptor.  Every check runs before anything is written, so after a refused
+ *     refit the previous scene renders exactly as before.  A CUDA failure part-way through
+ *     leaves no scene, like a failed rt_scene_upload.
+ *   - Like rt_scene_upload, it must not run while a render on another stream is in flight.
+ *   - The tree keeps the topology built for the uploaded scene; so does the split into the
+ *     primitives every ray tests and those in the LBVH.  Results never depend on the topology,
+ *     but the nodes a ray visits grow as the geometry moves away from what the tree was built
+ *     for; calling rt_scene_upload again rebuilds the tree.  A refit of the unchanged scene
+ *     rewrites the node array byte for byte.
+ *   - rt_stats after a refit: ms_upload = conversion and copies, ms_build = the refit kernels,
+ *     kernel_launches and scene_bytes_h2d = those of the refit. */
+int  rt_scene_refit(rt_context* ctx, const rt_scene* scene);
+
 /* ---- the hot path: Scene::renderScene ----------------------------------- */
 /* rgb: caller-owned double[height][width][3], row 0 = top (src/scene.cpp:26-31),
  * i.e. exactly Scene::RasterImage (src/scene.h:11).  Blocking.
