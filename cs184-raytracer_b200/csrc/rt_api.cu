@@ -18,7 +18,6 @@
 #include <chrono>
 #include <string>
 #include <thread>
-#include <type_traits>
 #include <vector>
 
 #include "rt_bvh.h"
@@ -118,6 +117,68 @@ struct TileLayout {
     }
 };
 
+// A device array of the scene: grow-only storage and the number of elements the scene holds in it.
+template <typename T>
+struct SceneArray : DevBuf<T> {
+    size_t used = 0;
+    cudaError_t hold(size_t count) { used = count; return this->ensure(count); }
+};
+
+// The scene an rt_context holds: its device arrays, the DScene that points into them, the LBVH bookkeeping of the
+// hit sort and the refit, and the structure rt_scene_refit requires unchanged.
+struct SceneStore {
+    DScene S{};
+    SceneArray<DGeom> geoms;
+    SceneArray<float4> sph_bound;
+    SceneArray<DMat> mats;
+    SceneArray<DLight> slights, alights;
+    SceneArray<double2> face_pts, face_nrm;
+    SceneArray<int> flat, all_prims;
+    SceneArray<BvhNode> nodes;
+    // Read only by the build and the refit, on the device that built the LBVH: its primitive codes and the wide
+    // level of every node slot.
+    DevBuf<int> bvh_prims, node_level;
+    size_t node_count = 0;
+    int bvh_levels = 0;
+    SortGrid sort_grid;                     // Morton grid over the LBVH primitives' centroid bounds
+    bool sort_ok = false;                   // scene has an LBVH (bounds known)
+    // Structure of the uploaded scene, which rt_scene_refit requires unchanged: (type, first_face, num_faces) per
+    // geometry, the face count and the FaceOwner table of k_pack_faces.  tri_pts: the six object-space points of
+    // every `tri` the device holds (a refit without faces derives the padding scale from them).
+    std::vector<int64_t> shape;
+    int64_t shape_faces = 0;
+    std::vector<FaceOwner> owners;
+    std::vector<double> tri_pts;
+
+    // Calls f(array, field) for every device array a render reads, as pointers to the SceneStore member and to the
+    // DScene field that points at it: the one list of them.  Stops at the first f that does not return RT_OK.
+    template <typename F>
+    static int each_array(F&& f) {
+        int rc = RT_OK;
+        auto go = [&](auto array, auto field) { if (rc == RT_OK) rc = f(array, field); };
+        go(&SceneStore::geoms, &DScene::geoms);
+        go(&SceneStore::sph_bound, &DScene::sph_bound);
+        go(&SceneStore::mats, &DScene::mats);
+        go(&SceneStore::slights, &DScene::slights);
+        go(&SceneStore::alights, &DScene::alights);
+        go(&SceneStore::face_pts, &DScene::face_pts);
+        go(&SceneStore::face_nrm, &DScene::face_nrm);
+        go(&SceneStore::flat, &DScene::flat);
+        go(&SceneStore::all_prims, &DScene::all_prims);
+        go(&SceneStore::nodes, &DScene::nodes);
+        return rc;
+    }
+
+    // Points S at the arrays of `from`: this store's own, or those of a store on the same device.  An array the
+    // scene holds nothing in stays null, so S.nodes is null without an LBVH.
+    void bind(const SceneStore& from) {
+        each_array([&](auto array, auto field) {
+            S.*field = (from.*array).used ? (from.*array).p : nullptr;
+            return RT_OK;
+        });
+    }
+};
+
 }  // namespace
 
 struct rt_context {
@@ -126,25 +187,7 @@ struct rt_context {
     cudaStream_t stream = nullptr;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
     bool have_scene = false;
-    // scene
-    DScene S;
-    DevBuf<DGeom> geoms;
-    DevBuf<DMat> mats;
-    DevBuf<DLight> slights, alights;
-    DevBuf<double2> face_pts, face_nrm;
-    DevBuf<int> flat, all_prims, bvh_prims;
-    DevBuf<float4> sph_bound;
-    DevBuf<BvhNode> nodes;
-    DevBuf<int> node_level;                 // wide level of every node slot (build_lbvh), for the refit
-    size_t node_count = 0;
-    int bvh_levels = 0;
-    // Structure of the uploaded scene, which rt_scene_refit requires unchanged: (type, first_face, num_faces) per
-    // geometry, the face count and the FaceOwner table of k_pack_faces.  tri_pts: the six object-space points of
-    // every `tri` the device holds (a refit without faces derives the padding scale from them).
-    std::vector<int64_t> shape;
-    int64_t shape_faces = 0;
-    std::vector<FaceOwner> owners;
-    std::vector<double> tri_pts;
+    SceneStore scene;
     DeviceArena scratch;                    // upload / LBVH-build temporaries
     // render state
     size_t cap = 0;                         // ray-queue capacity
@@ -165,8 +208,6 @@ struct rt_context {
     DevBuf<uint32_t> skeys[2];              // radix-sort ping-pong buffers
     DevBuf<int> svals[2];
     DevBuf<int> shist;
-    SortGrid sort_grid;                     // Morton grid over the LBVH primitives' centroid bounds
-    bool sort_ok = false;                   // scene has an LBVH (bounds known)
     cudaStream_t shadow_stream = nullptr;   // k_shadow of level l overlaps trace/shade of level l+1
     cudaEvent_t ev_hq_free[2] = {nullptr, nullptr};   // last k_shadow reading hit buffer b has been enqueued up to here
     cudaEvent_t ev_join = nullptr;
@@ -186,8 +227,6 @@ struct rt_context {
     // sub-context per additional device, each with a replica of the scene (see replicate_scene)
     std::vector<rt_context*> peers;
     bool peers_stale = true;                // scene uploaded since the peers were last synchronised
-    size_t used_geoms = 0, used_mats = 0, used_slights = 0, used_alights = 0, used_faces = 0, used_flat = 0,
-           used_all = 0, used_nodes = 0;
     int worker_rc = RT_OK;                  // result of the last worker-thread section (peers only)
     std::string worker_err;
     std::vector<void*> ipc_opened, ipc_created;
@@ -200,8 +239,7 @@ struct rt_context {
     std::vector<cudaEvent_t> evpool;        // RT_FLAG_TIME_KERNELS: (start, stop) pairs
     std::vector<int> evclass;
     size_t evused = 0;
-    size_t node_bytes = 0, face_bytes = 0;
-    rt_context() { memset(&S, 0, sizeof(S)); memset(&stats, 0, sizeof(stats)); }
+    rt_context() { memset(&stats, 0, sizeof(stats)); }
 };
 
 extern "C" {
@@ -484,75 +522,174 @@ size_t scene_scratch_bytes(const rt_scene* s, size_t n_owners, size_t n_simple, 
     return std::max(need_faces, lbvh_scratch_bytes(n_bvh));
 }
 
+// What an upload or a refit has enqueued: kernel launches and host-to-device bytes (counted by h2d).
+struct SceneWork {
+    int launches = 0;
+    size_t h2d_bytes = 0;
+};
+
+// A host-to-device copy of an upload or a refit, counted in its rt_stats.scene_bytes_h2d.
+cudaError_t h2d(SceneWork& w, void* dst, const void* src, size_t bytes, cudaStream_t st) {
+    if (!bytes) return cudaSuccess;
+    w.h2d_bytes += bytes;
+    return cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, st);
+}
+
 // Raw faces (host or device memory, see RT_SCENE_FACES_ON_DEVICE) -> the 80-byte face records and the FACE codes
 // of all_prims / bvh_prims (k_pack_faces).  Host faces are staged in ctx->scratch.
-int pack_faces(rt_context* ctx, const rt_scene* s, const std::vector<FaceOwner>& owners, int* launches) {
+int pack_faces(rt_context* ctx, const rt_scene* s, const std::vector<FaceOwner>& owners, SceneWork& w) {
     cudaStream_t st = ctx->stream;
+    SceneStore& sc = ctx->scene;
     const size_t nf = (size_t)s->num_faces;
     const double *raw_p = s->face_points, *raw_n = s->face_normals;
     if (!(s->flags & RT_SCENE_FACES_ON_DEVICE)) {
         double* up = ctx->scratch.take<double>(nf * 9);
         double* un = ctx->scratch.take<double>(nf * 9);
         if (!up || !un) return fail(RT_ERR_OOM, "upload scratch arena exhausted");
-        CU(cudaMemcpyAsync(up, s->face_points, sizeof(double) * 9 * nf, cudaMemcpyHostToDevice, st));
-        CU(cudaMemcpyAsync(un, s->face_normals, sizeof(double) * 9 * nf, cudaMemcpyHostToDevice, st));
+        CU(h2d(w, up, s->face_points, sizeof(double) * 9 * nf, st));
+        CU(h2d(w, un, s->face_normals, sizeof(double) * 9 * nf, st));
         raw_p = up; raw_n = un;
     }
     FaceOwner* d_owners = ctx->scratch.take<FaceOwner>(owners.size() ? owners.size() : 1);
     if (!d_owners) return fail(RT_ERR_OOM, "upload scratch arena exhausted");
-    if (!owners.empty())
-        CU(cudaMemcpyAsync(d_owners, owners.data(), sizeof(FaceOwner) * owners.size(), cudaMemcpyHostToDevice, st));
+    CU(h2d(w, d_owners, owners.data(), sizeof(FaceOwner) * owners.size(), st));
     k_pack_faces<<<(unsigned)((nf + 255) / 256), 256, 0, st>>>((long long)nf, raw_p, raw_n, d_owners, (int)owners.size(),
-                                                              ctx->face_pts.p, ctx->face_nrm.p, ctx->all_prims.p,
-                                                              ctx->bvh_prims.p);
-    (*launches)++;
+                                                              sc.face_pts.p, sc.face_nrm.p, sc.all_prims.p, sc.bvh_prims.p);
+    w.launches++;
     LAUNCHED("k_pack_faces", st);
     return RT_OK;
 }
 
-// The geometry, material and light tables to the device, and the DScene fields that point at them or count them
-// (the material and light counts may change between a scene and its refit).
-int upload_tables(rt_context* ctx, const rt_scene* s, const SceneConv& c) {
+// The geometry, material and light tables to the device, and the DScene fields that count them (the material and
+// light counts may change between a scene and its refit) and the camera.
+int upload_tables(rt_context* ctx, const rt_scene* s, const SceneConv& c, SceneWork& w) {
     cudaStream_t st = ctx->stream;
-    CU(ctx->geoms.ensure(c.geoms.size()));
-    CU(ctx->sph_bound.ensure(c.geoms.size()));
-    CU(ctx->mats.ensure(c.mats.size()));
-    CU(ctx->slights.ensure(c.slights.size()));
-    CU(ctx->alights.ensure(c.alights.size()));
-    if (!c.geoms.empty()) {
-        CU(cudaMemcpyAsync(ctx->geoms.p, c.geoms.data(), sizeof(DGeom) * c.geoms.size(), cudaMemcpyHostToDevice, st));
-        CU(cudaMemcpyAsync(ctx->sph_bound.p, c.sph_bound.data(), sizeof(float4) * c.sph_bound.size(), cudaMemcpyHostToDevice, st));
-    }
-    if (!c.mats.empty()) CU(cudaMemcpyAsync(ctx->mats.p, c.mats.data(), sizeof(DMat) * c.mats.size(), cudaMemcpyHostToDevice, st));
-    if (!c.slights.empty()) CU(cudaMemcpyAsync(ctx->slights.p, c.slights.data(), sizeof(DLight) * c.slights.size(), cudaMemcpyHostToDevice, st));
-    if (!c.alights.empty()) CU(cudaMemcpyAsync(ctx->alights.p, c.alights.data(), sizeof(DLight) * c.alights.size(), cudaMemcpyHostToDevice, st));
-    DScene& S = ctx->S;
+    SceneStore& sc = ctx->scene;
+    CU(sc.geoms.hold(c.geoms.size()));
+    CU(sc.sph_bound.hold(c.sph_bound.size()));
+    CU(sc.mats.hold(c.mats.size()));
+    CU(sc.slights.hold(c.slights.size()));
+    CU(sc.alights.hold(c.alights.size()));
+    CU(h2d(w, sc.geoms.p, c.geoms.data(), sizeof(DGeom) * c.geoms.size(), st));
+    CU(h2d(w, sc.sph_bound.p, c.sph_bound.data(), sizeof(float4) * c.sph_bound.size(), st));
+    CU(h2d(w, sc.mats.p, c.mats.data(), sizeof(DMat) * c.mats.size(), st));
+    CU(h2d(w, sc.slights.p, c.slights.data(), sizeof(DLight) * c.slights.size(), st));
+    CU(h2d(w, sc.alights.p, c.alights.data(), sizeof(DLight) * c.alights.size(), st));
+    DScene& S = sc.S;
     memcpy(&S.cam, &s->camera, sizeof(DCamera));
-    S.geoms = ctx->geoms.p;
-    S.sph_bound = ctx->sph_bound.p;
-    S.mats = ctx->mats.p;
-    S.slights = ctx->slights.p;
-    S.alights = ctx->alights.p;
     S.num_geoms = (int)c.geoms.size();
     S.num_slights = (int)c.slights.size();
     S.num_alights = (int)c.alights.size();
-    ctx->used_geoms = c.geoms.size(); ctx->used_mats = c.mats.size();
-    ctx->used_slights = c.slights.size(); ctx->used_alights = c.alights.size();
     return RT_OK;
 }
 
-// Bytes upload_tables copies.
-size_t table_bytes(const SceneConv& c) {
-    return sizeof(DGeom) * c.geoms.size() + sizeof(DMat) * c.mats.size() + sizeof(DLight) * (c.slights.size() + c.alights.size());
+// Where the primitives of a scene go, decided on the host before anything is written: reference order (all_prims),
+// then the flat / LBVH split.  Only the per-GEOMETRY bookkeeping is done here; the per-face arrays (geometry / local
+// index of a face, FACE codes in reference and LBVH order) are expanded on the device by k_pack_faces from the
+// FaceOwner table.
+struct ScenePlan {
+    std::vector<int> simple_all_pos;        // all_prims position of every sphere / `tri` code, geometry order
+    std::vector<FaceOwner> owners;          // sorted by first face; no two share a face
+    std::vector<int> flat_codes, bvh_codes; // bvh_codes: the spheres and `tri`s of the LBVH only
+    size_t n_all = 0, n_bvh = 0;
+    int group_sizes[2] = {0, 0};            // LBVH groups: those spheres and `tri`s, then the mesh faces
+    int group_first_code[2] = {0, 0};       // first primitive code of each group (all build_lbvh needs from the host side)
+    int single_leaf = 0;                    // an LBVH of exactly one primitive: its code
+};
+
+int plan_scene(const rt_scene* s, const SceneConv& c, ScenePlan& p) {
+    const std::vector<int>& simple_codes = c.simple_codes;
+    size_t n_mesh_faces = 0;
+    for (int i = 0; i < s->num_geometries; i++) {
+        const rt_geometry& g = s->geometries[i];
+        if (g.type == RT_GEOM_SPHERE || g.type == RT_GEOM_TRI) {
+            p.simple_all_pos.push_back((int)p.n_all);
+            p.n_all++;
+        }
+        if (g.type != RT_GEOM_SPHERE && g.num_faces > 0) {
+            FaceOwner o;
+            o.geom = i; o.first = (int)g.first_face; o.count = (int)g.num_faces;
+            o.all_off = g.type == RT_GEOM_MESH ? (int)p.n_all : -1;
+            o.bvh_off = g.type == RT_GEOM_MESH ? (int)n_mesh_faces : -1;     // + n_simple_in_bvh below
+            p.owners.push_back(o);
+        }
+        if (g.type == RT_GEOM_MESH) {
+            p.n_all += (size_t)g.num_faces;
+            n_mesh_faces += (size_t)g.num_faces;
+        }
+    }
+    if (p.n_all > (size_t)INT32_MAX) return fail(RT_ERR_INVALID, "too many primitives (%zu)", p.n_all);
+    int first_mesh_face_code = 0;
+    for (const FaceOwner& o : p.owners)
+        if (o.all_off >= 0) { first_mesh_face_code = (PRIM_FACE << PRIM_KIND_SHIFT) | o.first; break; }
+    std::vector<FaceOwner>& owners = p.owners;
+    std::sort(owners.begin(), owners.end(), [](const FaceOwner& a, const FaceOwner& b) { return a.first < b.first; });
+    for (size_t k = 1; k < owners.size(); k++)
+        if (owners[k].first < owners[k - 1].first + owners[k - 1].count)
+            return fail(RT_ERR_INVALID, "geometries %d and %d share faces", owners[k - 1].geom, owners[k].geom);
+    // spheres and `tri`s: few -> tested by every ray in reference order; many -> into the
+    // LBVH, except giants (floors) that would bloat its upper levels.
+    const size_t kFlatMax = 64, kGiantMax = 16;
+    if (simple_codes.size() <= kFlatMax) {
+        p.flat_codes = simple_codes;
+    } else {
+        double uext = 0;
+        for (int a = 0; a < 3; a++) uext = std::fmax(uext, c.simple_hi[a] - c.simple_lo[a]);
+        for (size_t k = 0; k < simple_codes.size(); k++) {
+            if (c.simple_ext[k] > 0.5 * uext && p.flat_codes.size() < kGiantMax) p.flat_codes.push_back(simple_codes[k]);
+            else p.bvh_codes.push_back(simple_codes[k]);
+        }
+    }
+    const int n_simple_in_bvh = (int)p.bvh_codes.size();
+    p.n_bvh = (size_t)n_simple_in_bvh + n_mesh_faces;
+    for (FaceOwner& o : owners)
+        if (o.bvh_off >= 0) o.bvh_off += n_simple_in_bvh;
+    p.group_sizes[0] = n_simple_in_bvh; p.group_sizes[1] = (int)n_mesh_faces;
+    p.group_first_code[0] = n_simple_in_bvh ? p.bvh_codes[0] : 0; p.group_first_code[1] = first_mesh_face_code;
+    p.single_leaf = p.n_bvh == 1 ? (n_simple_in_bvh ? p.bvh_codes[0] : first_mesh_face_code) : 0;
+    return RT_OK;
 }
 
-// Morton grid of the hit sort over the LBVH primitives' centroid bounds cb (min xyz, max xyz).
-void set_sort_grid(rt_context* ctx, const float* cb) {
+// The end of an upload or a refit, once its arrays are held and filled and ev1 is recorded: binds the DScene to the
+// arrays, builds the LBVH from the upload's plan, or refits the uploaded one when plan is null, applies its padding
+// scale and hit-sort grid, waits for the device, reports the times and counts, and makes the scene current.
+int commit_scene(rt_context* ctx, SceneConv& c, SceneWork& w, const ScenePlan* plan) {
+    SceneStore& sc = ctx->scene;
+    DScene& S = sc.S;
+    cudaStream_t st = ctx->stream;
+    sc.bind(sc);
+    float cb[6] = {0, 0, 0, 0, 0, 0}, pad_scale = 0.f;     // the LBVH primitives' centroid bounds (min xyz, max xyz)
+    if (S.nodes) {
+        const float extra_abs = std::nextafter((float)c.origin_abs, INFINITY);
+        char err[256] = "";
+        int brc = plan ? build_lbvh(S, sc.bvh_prims.p, plan->group_first_code, S.num_bvh_prims, plan->group_sizes, 2,
+                                    extra_abs, st, ctx->scratch, sc.nodes.p, &sc.node_count, &w.launches, err, sizeof(err),
+                                    cb, &pad_scale, sc.node_level.p, &sc.bvh_levels)
+                       : refit_lbvh(S, sc.bvh_prims.p, S.num_bvh_prims, sc.node_level.p, sc.bvh_levels, sc.node_count,
+                                    extra_abs, st, ctx->scratch, sc.nodes.p, &w.launches, err, sizeof(err), cb, &pad_scale);
+        ctx->scratch.reset();
+        if (brc != RT_OK) return fail(brc, "LBVH %s: %s", plan ? "build" : "refit", err);
+    }
+    S.origin_limit = S.nodes ? pad_scale : 3.0e38f;
+    // Morton grid of the hit sort over the centroid bounds; none without an LBVH
     float ext = 0.f;
     for (int a = 0; a < 3; a++) ext = fmaxf(ext, cb[3 + a] - cb[a]);
-    ctx->sort_ok = ext > 0.f && std::isfinite(ext);
-    for (int a = 0; a < 3; a++) ctx->sort_grid.lo[a] = cb[a];
-    ctx->sort_grid.scale = ctx->sort_ok ? 1024.f / ext : 0.f;
+    sc.sort_ok = ext > 0.f && std::isfinite(ext);
+    for (int a = 0; a < 3; a++) sc.sort_grid.lo[a] = cb[a];
+    sc.sort_grid.scale = sc.sort_ok ? 1024.f / ext : 0.f;
+    CU(cudaEventRecord(ctx->ev_build, st));
+    CU(cudaStreamSynchronize(st));
+    float ms0 = 0, ms1 = 0;
+    cudaEventElapsedTime(&ms0, ctx->ev0, ctx->ev1);
+    cudaEventElapsedTime(&ms1, ctx->ev1, ctx->ev_build);
+    sc.tri_pts = std::move(c.tri_pts);      // a refit without faces converted a copy of the ones kept
+    ctx->stats.ms_upload = ms0;
+    ctx->stats.ms_build = ms1;
+    ctx->stats.kernel_launches = (uint64_t)w.launches;
+    ctx->stats.scene_bytes_h2d = w.h2d_bytes;
+    ctx->have_scene = true;
+    ctx->peers_stale = true;
+    return RT_OK;
 }
 
 }  // namespace
@@ -565,160 +702,60 @@ int rt_scene_upload(rt_context* ctx, const rt_scene* s) {
     if (rc != RT_OK) return rc;
     CU(cudaSetDevice(ctx->device));
     ctx->have_scene = false;
-    ctx->sort_ok = false;
-    ctx->peers_stale = true;
     cudaStream_t st = ctx->stream;
     CU(cudaEventRecord(ctx->ev0, st));
-    int launches = 0;
-    const bool faces_on_device = (s->flags & RT_SCENE_FACES_ON_DEVICE) != 0;
-
-    // ---- host-side conversion of the small arrays ----
-    const int ng = s->num_geometries;
     SceneConv c;
     if ((rc = convert_scene(s, nullptr, c)) != RT_OK) return rc;
-    const std::vector<int>& simple_codes = c.simple_codes;
+    ScenePlan P;
+    if ((rc = plan_scene(s, c, P)) != RT_OK) return rc;
 
-    // ---- primitive codes: reference order, then the flat / BVH split ----
-    // Only the per-GEOMETRY bookkeeping is done here; the per-face arrays (geometry / local
-    // index of a face, FACE codes in reference and LBVH order) are expanded on the device by
-    // k_pack_faces from the FaceOwner table.
-    std::vector<int> simple_all_pos;
-    std::vector<FaceOwner> owners;
-    size_t n_all = 0, n_mesh_faces = 0;
-    for (int i = 0; i < ng; i++) {
-        const rt_geometry& g = s->geometries[i];
-        if (g.type == RT_GEOM_SPHERE || g.type == RT_GEOM_TRI) {
-            simple_all_pos.push_back((int)n_all);
-            n_all++;
-        }
-        if (g.type != RT_GEOM_SPHERE && g.num_faces > 0) {
-            FaceOwner o;
-            o.geom = i; o.first = (int)g.first_face; o.count = (int)g.num_faces;
-            o.all_off = g.type == RT_GEOM_MESH ? (int)n_all : -1;
-            o.bvh_off = g.type == RT_GEOM_MESH ? (int)n_mesh_faces : -1;     // + n_simple_in_bvh below
-            owners.push_back(o);
-        }
-        if (g.type == RT_GEOM_MESH) {
-            n_all += (size_t)g.num_faces;
-            n_mesh_faces += (size_t)g.num_faces;
-        }
-    }
-    if (n_all > (size_t)INT32_MAX) return fail(RT_ERR_INVALID, "too many primitives (%zu)", n_all);
-    int first_mesh_face_code = 0;
-    for (const FaceOwner& o : owners)
-        if (o.all_off >= 0) { first_mesh_face_code = (PRIM_FACE << PRIM_KIND_SHIFT) | o.first; break; }
-    std::sort(owners.begin(), owners.end(), [](const FaceOwner& a, const FaceOwner& b) { return a.first < b.first; });
-    for (size_t k = 1; k < owners.size(); k++)
-        if (owners[k].first < owners[k - 1].first + owners[k - 1].count)
-            return fail(RT_ERR_INVALID, "geometries %d and %d share faces", owners[k - 1].geom, owners[k].geom);
-    // spheres and `tri`s: few -> tested by every ray in reference order; many -> into the
-    // LBVH, except giants (floors) that would bloat its upper levels.
-    std::vector<int> flat_codes, bvh_codes;
-    const size_t kFlatMax = 64, kGiantMax = 16;
-    if (simple_codes.size() <= kFlatMax) {
-        flat_codes = simple_codes;
-    } else {
-        double uext = 0;
-        for (int a = 0; a < 3; a++) uext = std::fmax(uext, c.simple_hi[a] - c.simple_lo[a]);
-        for (size_t k = 0; k < simple_codes.size(); k++) {
-            if (c.simple_ext[k] > 0.5 * uext && flat_codes.size() < kGiantMax) flat_codes.push_back(simple_codes[k]);
-            else bvh_codes.push_back(simple_codes[k]);
-        }
-    }
-    const int n_simple_in_bvh = (int)bvh_codes.size();       // bvh_codes: the simple part only (host copy)
-    const size_t n_bvh = (size_t)n_simple_in_bvh + n_mesh_faces;
-    for (FaceOwner& o : owners)
-        if (o.bvh_off >= 0) o.bvh_off += n_simple_in_bvh;
-    const int group_sizes[2] = {n_simple_in_bvh, (int)n_mesh_faces};
-    // first primitive code of each LBVH group (all build_lbvh needs from the host side)
-    const int group_first_code[2] = {n_simple_in_bvh ? bvh_codes[0] : 0, first_mesh_face_code};
-
-    // ---- uploads ----
-    DScene& S = ctx->S;
+    // ---- device arrays, copies and the packing kernels ----
+    SceneStore& sc = ctx->scene;
+    DScene& S = sc.S;
     memset(&S, 0, sizeof(S));
-    if ((rc = upload_tables(ctx, s, c)) != RT_OK) return rc;
-    CU(ctx->flat.ensure(flat_codes.size()));
-    CU(ctx->all_prims.ensure(n_all));
-    CU(ctx->bvh_prims.ensure(n_bvh));
-    CU(ctx->face_pts.ensure((size_t)s->num_faces * RT_FACE_D2));
-    CU(ctx->face_nrm.ensure((size_t)s->num_faces * RT_FACE_D2));
-    if (!flat_codes.empty()) CU(cudaMemcpyAsync(ctx->flat.p, flat_codes.data(), sizeof(int) * flat_codes.size(), cudaMemcpyHostToDevice, st));
-    if (!bvh_codes.empty()) CU(cudaMemcpyAsync(ctx->bvh_prims.p, bvh_codes.data(), sizeof(int) * bvh_codes.size(), cudaMemcpyHostToDevice, st));
+    SceneWork w;
+    if ((rc = upload_tables(ctx, s, c, w)) != RT_OK) return rc;
+    const size_t nf = (size_t)s->num_faces;
+    CU(sc.flat.hold(P.flat_codes.size()));
+    CU(sc.all_prims.hold(P.n_all));
+    CU(sc.bvh_prims.ensure(P.n_bvh));
+    CU(sc.face_pts.hold(nf * RT_FACE_D2));
+    CU(sc.face_nrm.hold(nf * RT_FACE_D2));
+    CU(h2d(w, sc.flat.p, P.flat_codes.data(), sizeof(int) * P.flat_codes.size(), st));
+    CU(h2d(w, sc.bvh_prims.p, P.bvh_codes.data(), sizeof(int) * P.bvh_codes.size(), st));
     // one arena reservation covers the raw-face staging and (afterwards, reused) the LBVH build
-    CU(ctx->scratch.reserve(scene_scratch_bytes(s, owners.size(), simple_codes.size(), n_bvh)));
+    const std::vector<int>& simple_codes = c.simple_codes;
+    CU(ctx->scratch.reserve(scene_scratch_bytes(s, P.owners.size(), simple_codes.size(), P.n_bvh)));
     if (!simple_codes.empty()) {
         int* d_pos = ctx->scratch.take<int>(simple_codes.size());
         int* d_code = ctx->scratch.take<int>(simple_codes.size());
         if (!d_pos || !d_code) return fail(RT_ERR_OOM, "upload scratch arena exhausted");
-        CU(cudaMemcpyAsync(d_pos, simple_all_pos.data(), sizeof(int) * simple_codes.size(), cudaMemcpyHostToDevice, st));
-        CU(cudaMemcpyAsync(d_code, simple_codes.data(), sizeof(int) * simple_codes.size(), cudaMemcpyHostToDevice, st));
+        CU(h2d(w, d_pos, P.simple_all_pos.data(), sizeof(int) * simple_codes.size(), st));
+        CU(h2d(w, d_code, simple_codes.data(), sizeof(int) * simple_codes.size(), st));
         k_scatter_codes<<<(unsigned)((simple_codes.size() + 255) / 256), 256, 0, st>>>((int)simple_codes.size(), d_pos, d_code,
-                                                                                    ctx->all_prims.p);
-        launches++;
+                                                                                    sc.all_prims.p);
+        w.launches++;
         LAUNCHED("k_scatter_codes", st);
     }
-    if (s->num_faces && (rc = pack_faces(ctx, s, owners, &launches)) != RT_OK) return rc;
+    if (nf && (rc = pack_faces(ctx, s, P.owners, w)) != RT_OK) return rc;
     CU(cudaStreamSynchronize(st));
     ctx->scratch.reset();
-
-    S.face_pts = ctx->face_pts.p;
-    S.face_nrm = ctx->face_nrm.p;
-    S.flat = ctx->flat.p;
-    S.all_prims = ctx->all_prims.p;
-    S.num_flat = (int)flat_codes.size();
-    S.num_all = (int)n_all;
-    S.num_bvh_prims = (int)n_bvh;
-    S.single_leaf = n_bvh == 1 ? (n_simple_in_bvh ? bvh_codes[0] : first_mesh_face_code) : 0;
+    S.num_flat = (int)P.flat_codes.size();
+    S.num_all = (int)P.n_all;
+    S.num_bvh_prims = (int)P.n_bvh;
+    S.single_leaf = P.single_leaf;
     CU(cudaEventRecord(ctx->ev1, st));
-
-    // ---- LBVH ----
-    cudaEvent_t evb = ctx->ev_build;
-    size_t node_count = 0;
-    int levels = 0;
-    S.origin_limit = 3.0e38f;
-    if (n_bvh >= 2) {
-        const float extra_abs = std::nextafter((float)c.origin_abs, INFINITY);
-        char err[256] = "";
-        float cb[6] = {0, 0, 0, 0, 0, 0};
-        float pad_scale = 0.f;
-        CU(ctx->nodes.ensure(n_bvh + 2));
-        CU(ctx->node_level.ensure(n_bvh + 2));
-        int brc = build_lbvh(S, ctx->bvh_prims.p, group_first_code, (int)n_bvh, group_sizes, 2, extra_abs, st,
-                             ctx->scratch, ctx->nodes.p, &node_count, &launches, err, sizeof(err), cb, &pad_scale,
-                             ctx->node_level.p, &levels);
-        ctx->scratch.reset();
-        if (brc != RT_OK) return fail(brc, "LBVH build: %s", err);
-        S.origin_limit = pad_scale;
-        set_sort_grid(ctx, cb);
+    sc.nodes.used = sc.node_count = 0;
+    if (P.n_bvh >= 2) {
+        CU(sc.nodes.hold(P.n_bvh + 2));
+        CU(sc.node_level.ensure(P.n_bvh + 2));
     }
-    S.nodes = node_count ? ctx->nodes.p : nullptr;
-    cudaEventRecord(evb, st);
-    CU(cudaStreamSynchronize(st));
-    float ms0 = 0, ms1 = 0;
-    cudaEventElapsedTime(&ms0, ctx->ev0, ctx->ev1);
-    cudaEventElapsedTime(&ms1, ctx->ev1, evb);
-    ctx->used_faces = (size_t)s->num_faces; ctx->used_flat = flat_codes.size(); ctx->used_all = n_all;
-    ctx->used_nodes = node_count ? n_bvh + 2 : 0;
-    ctx->node_count = node_count;
-    ctx->bvh_levels = levels;
-    ctx->node_bytes = sizeof(BvhNode) * node_count;
-    ctx->face_bytes = sizeof(double2) * RT_FACE_D2 * 2 * (size_t)s->num_faces;
-    ctx->shape_faces = s->num_faces;
-    ctx->shape.resize(3 * (size_t)ng);
-    for (int i = 0; i < ng; i++) {
-        ctx->shape[3 * (size_t)i] = s->geometries[i].type;
-        ctx->shape[3 * (size_t)i + 1] = s->geometries[i].first_face;
-        ctx->shape[3 * (size_t)i + 2] = s->geometries[i].num_faces;
-    }
-    ctx->owners = owners;
-    ctx->tri_pts = std::move(c.tri_pts);
-    ctx->stats.scene_bytes_h2d = table_bytes(c) + sizeof(int) * (flat_codes.size() + 2 * simple_codes.size() + bvh_codes.size()) +
-                                 sizeof(FaceOwner) * owners.size() + (faces_on_device ? 0 : (size_t)s->num_faces * (2 * 72));
-    ctx->stats.ms_upload = ms0;
-    ctx->stats.ms_build = ms1;
-    ctx->stats.kernel_launches = (uint64_t)launches;
-    ctx->have_scene = true;
-    return RT_OK;
+    sc.shape_faces = s->num_faces;
+    sc.shape.clear();
+    for (int i = 0; i < s->num_geometries; i++)
+        sc.shape.insert(sc.shape.end(), {s->geometries[i].type, s->geometries[i].first_face, s->geometries[i].num_faces});
+    sc.owners = std::move(P.owners);
+    return commit_scene(ctx, c, w, &P);
 }
 
 int rt_scene_refit(rt_context* ctx, const rt_scene* s) {
@@ -730,16 +767,17 @@ int rt_scene_refit(rt_context* ctx, const rt_scene* s) {
     const bool keep_faces = s && s->face_points == nullptr;
     int rc = validate_scene(s, keep_faces);
     if (rc != RT_OK) return rc;
+    SceneStore& sc = ctx->scene;
     const int ng = s->num_geometries;
-    if ((size_t)ng * 3 != ctx->shape.size())
+    if ((size_t)ng * 3 != sc.shape.size())
         return fail(RT_ERR_INVALID, "rt_scene_refit: num_geometries %d differs from the uploaded scene's %zu", ng,
-                    ctx->shape.size() / 3);
-    if (s->num_faces != ctx->shape_faces)
+                    sc.shape.size() / 3);
+    if (s->num_faces != sc.shape_faces)
         return fail(RT_ERR_INVALID, "rt_scene_refit: num_faces %lld differs from the uploaded scene's %lld",
-                    (long long)s->num_faces, (long long)ctx->shape_faces);
+                    (long long)s->num_faces, (long long)sc.shape_faces);
     for (int i = 0; i < ng; i++) {
         const rt_geometry& g = s->geometries[i];
-        const int64_t* u = ctx->shape.data() + 3 * (size_t)i;
+        const int64_t* u = sc.shape.data() + 3 * (size_t)i;
         const int64_t got[3] = {g.type, g.first_face, g.num_faces};
         static const char* const field[3] = {"type", "first_face", "num_faces"};
         for (int f = 0; f < 3; f++)
@@ -749,46 +787,20 @@ int rt_scene_refit(rt_context* ctx, const rt_scene* s) {
     }
     CU(cudaSetDevice(ctx->device));
     SceneConv c;
-    if ((rc = convert_scene(s, keep_faces ? &ctx->tri_pts : nullptr, c)) != RT_OK) return rc;
+    if ((rc = convert_scene(s, keep_faces ? &sc.tri_pts : nullptr, c)) != RT_OK) return rc;
 
     // ---- writes: from here a failure leaves no scene, like a failed upload ----
     ctx->have_scene = false;
-    ctx->peers_stale = true;
     cudaStream_t st = ctx->stream;
     CU(cudaEventRecord(ctx->ev0, st));
-    int launches = 0;
-    if ((rc = upload_tables(ctx, s, c)) != RT_OK) return rc;
-    DScene& S = ctx->S;
+    SceneWork w;
+    if ((rc = upload_tables(ctx, s, c, w)) != RT_OK) return rc;
     // the upload reserved this much already: no allocation
-    CU(ctx->scratch.reserve(scene_scratch_bytes(s, ctx->owners.size(), c.simple_codes.size(), (size_t)S.num_bvh_prims)));
-    if (!keep_faces && s->num_faces && (rc = pack_faces(ctx, s, ctx->owners, &launches)) != RT_OK) return rc;
+    CU(ctx->scratch.reserve(scene_scratch_bytes(s, sc.owners.size(), c.simple_codes.size(), (size_t)sc.S.num_bvh_prims)));
+    if (!keep_faces && s->num_faces && (rc = pack_faces(ctx, s, sc.owners, w)) != RT_OK) return rc;
     ctx->scratch.reset();       // the refit's launches are stream-ordered after k_pack_faces: the staging is free
     CU(cudaEventRecord(ctx->ev1, st));
-    if (S.nodes) {
-        const float extra_abs = std::nextafter((float)c.origin_abs, INFINITY);
-        char err[256] = "";
-        float cb[6], pad_scale = 0.f;
-        int brc = refit_lbvh(S, ctx->bvh_prims.p, S.num_bvh_prims, ctx->node_level.p, ctx->bvh_levels, ctx->node_count,
-                             extra_abs, st, ctx->scratch, ctx->nodes.p, &launches, err, sizeof(err), cb, &pad_scale);
-        ctx->scratch.reset();
-        if (brc != RT_OK) return fail(brc, "LBVH refit: %s", err);
-        S.origin_limit = pad_scale;
-        set_sort_grid(ctx, cb);
-    }
-    CU(cudaEventRecord(ctx->ev_build, st));
-    CU(cudaStreamSynchronize(st));
-    float ms0 = 0, ms1 = 0;
-    cudaEventElapsedTime(&ms0, ctx->ev0, ctx->ev1);
-    cudaEventElapsedTime(&ms1, ctx->ev1, ctx->ev_build);
-    if (!keep_faces) ctx->tri_pts = std::move(c.tri_pts);
-    ctx->stats.scene_bytes_h2d = table_bytes(c) + sizeof(float4) * c.sph_bound.size() +
-                                 (keep_faces ? 0 : sizeof(FaceOwner) * ctx->owners.size()) +
-                                 (keep_faces || (s->flags & RT_SCENE_FACES_ON_DEVICE) ? 0 : (size_t)s->num_faces * (2 * 72));
-    ctx->stats.ms_upload = ms0;
-    ctx->stats.ms_build = ms1;
-    ctx->stats.kernel_launches = (uint64_t)launches;
-    ctx->have_scene = true;
-    return RT_OK;
+    return commit_scene(ctx, c, w, nullptr);
 }
 
 }  // extern "C"
@@ -888,7 +900,7 @@ void release_queue(rt_context* ctx, int qi) { ctx->qpool[(size_t)qi].busy = fals
 template <bool BRUTE, bool COUNT, bool PRIMARY = false>
 int launch_trace(RenderJob& J, RayQ q, size_t off, int n, size_t nfront, HitQ h, unsigned long long* lc) {
     LaunchTimer lt(J, 0);
-    k_trace<BRUTE, COUNT, PRIMARY><<<(n + RT_BLOCK - 1) / RT_BLOCK, RT_BLOCK, 0, J.st>>>(J.ctx->S, q, off, n, nfront, h, lc,
+    k_trace<BRUTE, COUNT, PRIMARY><<<(n + RT_BLOCK - 1) / RT_BLOCK, RT_BLOCK, 0, J.st>>>(J.ctx->scene.S, q, off, n, nfront, h, lc,
                                                                                      J.ids_geom, J.ids_face, J.primary);
     J.launches++;
     LAUNCHED("k_trace", J.st);
@@ -896,10 +908,10 @@ int launch_trace(RenderJob& J, RayQ q, size_t off, int n, size_t nfront, HitQ h,
 }
 template <bool BRUTE, bool COUNT>
 int launch_shadow(RenderJob& J, int n, HitQ h, unsigned long long* lc, cudaStream_t st) {
-    unsigned long long threads = (unsigned long long)n * (unsigned)J.ctx->S.num_slights;
+    unsigned long long threads = (unsigned long long)n * (unsigned)J.ctx->scene.S.num_slights;
     if (!threads) return RT_OK;
     LaunchTimer lt(J, 2, st);
-    k_shadow<BRUTE, COUNT><<<(unsigned)((threads + RT_BLOCK - 1) / RT_BLOCK), RT_BLOCK, 0, st>>>(J.ctx->S, h, lc, J.ctx->fb.p);
+    k_shadow<BRUTE, COUNT><<<(unsigned)((threads + RT_BLOCK - 1) / RT_BLOCK), RT_BLOCK, 0, st>>>(J.ctx->scene.S, h, lc, J.ctx->fb.p);
     J.launches++;
     LAUNCHED("k_shadow", st);
     return RT_OK;
@@ -976,7 +988,7 @@ int process_levels(RenderJob& J, int q0, size_t n) {
             const unsigned sb = (unsigned)((m + 255) / 256);
             uint32_t *kin = ctx->skeys[0].p, *kout = ctx->skeys[1].p;
             int *vin = ctx->svals[0].p, *vout = ctx->svals[1].p;
-            k_hit_keys<<<sb, 256, 0, J.st>>>(ht, lc, ctx->sort_grid, kin, vin);
+            k_hit_keys<<<sb, 256, 0, J.st>>>(ht, lc, ctx->scene.sort_grid, kin, vin);
             int nl = 0;
             sort_pairs(J.st, kin, kout, vin, vout, ctx->shist.p, m, lc + CTR_HITS, &nl);
             sorted_order = vin;                 // k_shade gathers through it and writes the sorted queue
@@ -1005,7 +1017,7 @@ int process_levels(RenderJob& J, int q0, size_t n) {
         {
             LaunchTimer lt(J, 1);
             k_shade<<<(unsigned)((m + RT_SHADE_BLOCK - 1) / RT_SHADE_BLOCK), RT_SHADE_BLOCK, 0, J.st>>>(
-                ctx->S, sorted_order ? ht : h, h, sorted_order, lc, next, ctx->fb.p);
+                ctx->scene.S, sorted_order ? ht : h, h, sorted_order, lc, next, ctx->fb.p);
         }
         J.launches++;
         LAUNCHED("k_shade", J.st);
@@ -1025,7 +1037,7 @@ int process_levels(RenderJob& J, int q0, size_t n) {
         CU(cudaStreamSynchronize(ctx->copy_stream));
         const unsigned long long nhits = h_counts[0], nrefl = h_counts[1], nnext = nrefl + h_counts[2];
         ctx->stats.hits += nhits;
-        ctx->stats.rays_shadow += nhits * (unsigned long long)ctx->S.num_slights;
+        ctx->stats.rays_shadow += nhits * (unsigned long long)ctx->scene.S.num_slights;
         ctx->stats.rays_secondary += nnext;
         if (level == 0) progress_tick(J, 0.5 * (double)(off + (size_t)m) / (double)e.n);
         else progress_tick(J, 1.0 - 0.5 / (double)(level + 1));
@@ -1104,7 +1116,7 @@ int render_core(rt_context* ctx, const rt_params* p, cudaStream_t st, bool ids_o
         // RT_HIT_SORT_MIN_RAYS lowers the level size from which it is worth its launches (tests: 1).
         const char* mr = getenv("RT_HIT_SORT_MIN_RAYS");
         J.sort_min_rays = mr ? (size_t)atoll(mr) : 262144;
-        J.sort = ctx->sort_ok && !J.brute && p->bounce_depth >= 1 && !ids_only && !p->intersection_only;
+        J.sort = ctx->scene.sort_ok && !J.brute && p->bounce_depth >= 1 && !ids_only && !p->intersection_only;
     }
     if (J.sort) {
         CU(ctx->hsf.ensure(13 * maxchunk));
@@ -1167,7 +1179,7 @@ int render_core(rt_context* ctx, const rt_params* p, cudaStream_t st, bool ids_o
             if (rc != RT_OK) return rc;
             {
                 LaunchTimer lt(J, 3);
-                k_raygen<<<(n + RT_BLOCK - 1) / RT_BLOCK, RT_BLOCK, 0, st>>>(ctx->S, J.primary, n, pool_queue(ctx, q0));
+                k_raygen<<<(n + RT_BLOCK - 1) / RT_BLOCK, RT_BLOCK, 0, st>>>(ctx->scene.S, J.primary, n, pool_queue(ctx, q0));
             }
             J.launches++;
             LAUNCHED("k_raygen", st);
@@ -1294,48 +1306,33 @@ int ensure_peers(rt_context* ctx, int n) {
     return RT_OK;
 }
 
-// Device-to-device copy of the primary's scene arrays (faces, LBVH nodes, geometry/material/light tables) into
-// every sub-context: the LBVH is built once, not once per GPU.
+// Copies the primary's scene into every sub-context: the scalar state, then, for a sub-context on another device,
+// every scene array with a peer copy (the LBVH is built once, not once per GPU).  A sub-context on the primary's own
+// device reads the primary's arrays.
 int replicate_scene(rt_context* ctx, int n) {
     if (!ctx->peers_stale) return RT_OK;
     CU(cudaSetDevice(ctx->device));
+    const SceneStore& src = ctx->scene;
     for (int k = 0; k < n - 1; k++) {
         rt_context* pc = ctx->peers[(size_t)k];
-        if (pc->device == ctx->device) {      // sub-context on the primary's own device: same arrays, no copy
-            pc->S = ctx->S;
-            pc->sort_grid = ctx->sort_grid;
-            pc->sort_ok = ctx->sort_ok;
-            pc->node_bytes = ctx->node_bytes; pc->face_bytes = ctx->face_bytes;
-            pc->have_scene = true;
-            continue;
+        SceneStore& dst = pc->scene;
+        dst.S = src.S;
+        dst.sort_grid = src.sort_grid;
+        dst.sort_ok = src.sort_ok;
+        const bool same_device = pc->device == ctx->device;
+        if (!same_device) {
+            int rc = SceneStore::each_array([&](auto array, auto) -> int {
+                auto& to = dst.*array;
+                const auto& from = src.*array;
+                CU(cudaSetDevice(pc->device));
+                CU(to.hold(from.used));
+                CU(cudaSetDevice(ctx->device));
+                if (from.used) CU(cudaMemcpyPeerAsync(to.p, pc->device, from.p, ctx->device, sizeof(*from.p) * from.used, ctx->stream));
+                return RT_OK;
+            });
+            if (rc != RT_OK) return rc;
         }
-        auto copy = [&](auto& dst, const auto& src, size_t count) -> int {
-            using T = std::remove_pointer_t<decltype(src.p)>;
-            CU(cudaSetDevice(pc->device));
-            CU(dst.ensure(count));
-            CU(cudaSetDevice(ctx->device));
-            if (count) CU(cudaMemcpyPeerAsync(dst.p, pc->device, src.p, ctx->device, sizeof(T) * count, ctx->stream));
-            return RT_OK;
-        };
-        int rc;
-        if ((rc = copy(pc->geoms, ctx->geoms, ctx->used_geoms)) != RT_OK) return rc;
-        if ((rc = copy(pc->mats, ctx->mats, ctx->used_mats)) != RT_OK) return rc;
-        if ((rc = copy(pc->slights, ctx->slights, ctx->used_slights)) != RT_OK) return rc;
-        if ((rc = copy(pc->alights, ctx->alights, ctx->used_alights)) != RT_OK) return rc;
-        if ((rc = copy(pc->sph_bound, ctx->sph_bound, ctx->used_geoms)) != RT_OK) return rc;
-        if ((rc = copy(pc->face_pts, ctx->face_pts, ctx->used_faces * RT_FACE_D2)) != RT_OK) return rc;
-        if ((rc = copy(pc->face_nrm, ctx->face_nrm, ctx->used_faces * RT_FACE_D2)) != RT_OK) return rc;
-        if ((rc = copy(pc->flat, ctx->flat, ctx->used_flat)) != RT_OK) return rc;
-        if ((rc = copy(pc->all_prims, ctx->all_prims, ctx->used_all)) != RT_OK) return rc;
-        if ((rc = copy(pc->nodes, ctx->nodes, ctx->used_nodes)) != RT_OK) return rc;
-        pc->S = ctx->S;
-        pc->S.geoms = pc->geoms.p; pc->S.mats = pc->mats.p; pc->S.slights = pc->slights.p; pc->S.alights = pc->alights.p;
-        pc->S.sph_bound = pc->sph_bound.p; pc->S.face_pts = pc->face_pts.p; pc->S.face_nrm = pc->face_nrm.p;
-        pc->S.flat = pc->flat.p; pc->S.all_prims = pc->all_prims.p;
-        pc->S.nodes = ctx->S.nodes ? pc->nodes.p : nullptr;
-        pc->sort_grid = ctx->sort_grid;
-        pc->sort_ok = ctx->sort_ok;
-        pc->node_bytes = ctx->node_bytes; pc->face_bytes = ctx->face_bytes;
+        dst.bind(same_device ? src : dst);
         pc->have_scene = true;
     }
     CU(cudaStreamSynchronize(ctx->stream));
@@ -1693,10 +1690,10 @@ int rt_cast_rays(rt_context* ctx, int64_t n, const double* org, const double* di
     }
     const unsigned blocks = (unsigned)((N + RT_BLOCK - 1) / RT_BLOCK);
     if (flags & RT_FLAG_BRUTE_FORCE)
-        k_query<true><<<blocks, RT_BLOCK, 0, ctx->stream>>>(ctx->S, n, d_org.p, d_dir.p, reverse ? d_rev.p : nullptr, d_geom.p,
+        k_query<true><<<blocks, RT_BLOCK, 0, ctx->stream>>>(ctx->scene.S, n, d_org.p, d_dir.p, reverse ? d_rev.p : nullptr, d_geom.p,
                                                            d_face.p, d_dist.p, d_point.p, d_normal.p);
     else
-        k_query<false><<<blocks, RT_BLOCK, 0, ctx->stream>>>(ctx->S, n, d_org.p, d_dir.p, reverse ? d_rev.p : nullptr, d_geom.p,
+        k_query<false><<<blocks, RT_BLOCK, 0, ctx->stream>>>(ctx->scene.S, n, d_org.p, d_dir.p, reverse ? d_rev.p : nullptr, d_geom.p,
                                                             d_face.p, d_dist.p, d_point.p, d_normal.p);
     CU(cudaGetLastError());
     CU(cudaStreamSynchronize(ctx->stream));
@@ -1734,8 +1731,9 @@ int rt_divide_device(rt_context* ctx, double* d_values, int64_t count, double di
 
 int rt_scene_device_bytes(rt_context* ctx, uint64_t* node_bytes, uint64_t* face_bytes) {
     if (!ctx) return fail(RT_ERR_INVALID, "context is NULL");
-    if (node_bytes) *node_bytes = ctx->node_bytes;
-    if (face_bytes) *face_bytes = ctx->face_bytes;
+    const SceneStore& sc = ctx->scene;
+    if (node_bytes) *node_bytes = sizeof(BvhNode) * sc.node_count;
+    if (face_bytes) *face_bytes = sizeof(double2) * (sc.face_pts.used + sc.face_nrm.used);
     return RT_OK;
 }
 
@@ -1769,18 +1767,18 @@ int rt_microbench_gather(rt_context* ctx, uint64_t array_bytes, int loads_per_th
 int rt_microbench_node_walk(rt_context* ctx, int group, int visits_per_thread, double* visits_per_s, double* bytes_per_s) {
     if (!ctx || !visits_per_s || visits_per_thread < 1 || group < 1 || group > 32 || (group & (group - 1)))
         return fail(RT_ERR_INVALID, "rt_microbench_node_walk: bad argument (group must be a power of two <= 32)");
-    if (!ctx->have_scene || !ctx->S.nodes) return fail(RT_ERR_NO_SCENE, "rt_microbench_node_walk needs an uploaded scene with an LBVH");
+    if (!ctx->have_scene || !ctx->scene.S.nodes) return fail(RT_ERR_NO_SCENE, "rt_microbench_node_walk needs an uploaded scene with an LBVH");
     CU(cudaSetDevice(ctx->device));
     DevBuf<float> sink;
     CU(sink.ensure(1));
     // the traversal kernels' shape: 64-thread blocks, 16 resident per SM; 8 waves of them
     const int blocks = ctx->num_sms * RT_SHADOW_MINBLOCKS * 8;
-    k_node_walk<<<blocks, RT_BLOCK, 0, ctx->stream>>>(ctx->S.nodes, visits_per_thread, group, sink.p);   // warm-up
+    k_node_walk<<<blocks, RT_BLOCK, 0, ctx->stream>>>(ctx->scene.S.nodes, visits_per_thread, group, sink.p);   // warm-up
     LAUNCHED("k_node_walk", ctx->stream);
     float best = 1e30f;
     for (int rep = 0; rep < 5; rep++) {
         CU(cudaEventRecord(ctx->ev0, ctx->stream));
-        k_node_walk<<<blocks, RT_BLOCK, 0, ctx->stream>>>(ctx->S.nodes, visits_per_thread, group, sink.p);
+        k_node_walk<<<blocks, RT_BLOCK, 0, ctx->stream>>>(ctx->scene.S.nodes, visits_per_thread, group, sink.p);
         CU(cudaEventRecord(ctx->ev1, ctx->stream));
         CU(cudaStreamSynchronize(ctx->stream));
         float ms = 0;

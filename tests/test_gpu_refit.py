@@ -458,12 +458,18 @@ def test_refit_cost(pkg, gpu_renderer, tmp_path):
     t = pkg.HostScene.load(scene_path("inputs/input-02.rti"))
     s = C.cast(t.flat, C.POINTER(pkg.rt_scene)).contents
     r.upload(t)
-    upload_launches = r.stats()["kernel_launches"]
+    upload = r.stats()
     r.refit(t)
     with_faces = r.stats()
     r.refit(Desc(pkg, t.flat, t).without_faces().ptr)
     without = r.stats()
-    assert with_faces["kernel_launches"] == without["kernel_launches"] + 1 < upload_launches
+    assert with_faces["kernel_launches"] == without["kernel_launches"] + 1 < upload["kernel_launches"]
     owners = sum(1 for i in range(s.num_geometries) if s.geometries[i].num_faces > 0)
     assert with_faces["scene_bytes_h2d"] - without["scene_bytes_h2d"] == 144 * s.num_faces + 20 * owners
     assert without["scene_bytes_h2d"] < 144 * s.num_faces
+    # Only the upload sends primitive codes (4 B each): the flat list, the all_prims position and code of every sphere
+    # and `tri`, and those in the LBVH.  Up to 64 of them all go to the flat list.
+    simple = sum(1 for i in range(s.num_geometries) if s.geometries[i].type != pkg.binding.RT_GEOM_MESH)
+    assert 0 < simple <= 64
+    flat, simple_in_bvh = simple, 0
+    assert upload["scene_bytes_h2d"] - with_faces["scene_bytes_h2d"] == 4 * (flat + 2 * simple + simple_in_bvh)
