@@ -1222,6 +1222,9 @@ int render_core(rt_context* ctx, const rt_params* p, cudaStream_t st, bool ids_o
     for (int l = 0; l < used_levels; l++) {
         const unsigned long long* c = ctx->h_ctr + 4 + (size_t)l * CTR_COUNT;
         stats.degenerate_rays += c[CTR_DEGENERATE];
+        // process_levels counted hits x lights shadow rays; a light exactly at the hit point gives no ray (the
+        // reference would abort on it), so it is only a degenerate ray, as a degenerate secondary ray is
+        stats.rays_shadow -= c[CTR_S_DEGENERATE];
         stats.nodes_fetched[0] += c[CTR_NODES];
         stats.tris_tested[0] += c[CTR_TRIS];
         stats.spheres_tested[0] += c[CTR_SPHERES];

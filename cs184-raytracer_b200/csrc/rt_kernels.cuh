@@ -62,6 +62,7 @@ enum {
     CTR_DEGENERATE = 0,
     CTR_S_CULLED = 1,                                      // shadow rays answered without a traversal (COUNT builds)
     CTR_NODES = 2, CTR_TRIS = 3, CTR_SPHERES = 4,          // closest-hit kernel
+    CTR_S_DEGENERATE = 5,                                  // the shadow rays among CTR_DEGENERATE: not cast, so not in rays_shadow
     CTR_HITS = 6, CTR_NEXT = 7,                            // the last two words of the first line
     CTR_NEXT_T = 8,                                        // refracted children (stored from the END of the next queue)
     CTR_S_NODES = 9, CTR_S_TRIS = 10, CTR_S_SPHERES = 11,  // shadow kernel
@@ -414,6 +415,7 @@ __global__ void __launch_bounds__(RT_BLOCK, RT_SHADOW_MINBLOCKS) k_shadow(DScene
         d3 toL = point ? lv - P : -lv;                        // src/lights.h:34-37,50-53
         if (toL.x == 0 && toL.y == 0 && toL.z == 0) {
             atomicAdd(ctr + CTR_DEGENERATE, 1ull);            // reference would abort (src/rtbase.h:19-20)
+            atomicAdd(ctr + CTR_S_DEGENERATE, 1ull);          // the host takes it back out of rays_shadow
         } else {
             d3 L = ray_normalize(toL);
             double ndl = dot4(N, L);
@@ -424,7 +426,7 @@ __global__ void __launch_bounds__(RT_BLOCK, RT_SHADOW_MINBLOCKS) k_shadow(DScene
             // The Phong terms of this light (src/scene.cpp:95-106) BEFORE the occlusion query: when both are exactly
             // zero (light behind the surface and no specular lobe towards the viewer) the light adds +0 whether or not
             // it is occluded, so the query's answer cannot reach the frame and the traversal is skipped.  The
-            // reference casts that shadow ray too; it is still counted (rays_shadow = hits x lights on the host).
+            // reference casts that shadow ray too; it is still counted (rays_shadow = hits x lights - degenerate ones).
             const DMat* m = S.mats + S.geoms[h.geom[j]].mat;
             d3 V = mk3(h.fld(6, j), h.fld(7, j), h.fld(8, j));
             double att[3];

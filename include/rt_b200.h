@@ -167,7 +167,8 @@ typedef void (*rt_progress_fn)(int complete, int total, void* user);
 /* Ray/work statistics of the last render (a "ray" == one reference castRay call). */
 typedef struct rt_stats {
     uint64_t rays_primary;     /* src/scene.cpp:65 from :31                   */
-    uint64_t rays_shadow;      /* src/scene.cpp:91                            */
+    uint64_t rays_shadow;      /* src/scene.cpp:91: hits x non-ambient lights, less the degenerate ones (a point light
+                                  exactly at the hit point: counted in degenerate_rays only, as secondary rays are) */
     uint64_t rays_secondary;   /* src/scene.cpp:127,134                       */
     uint64_t degenerate_rays;  /* rays the reference would have aborted on (src/rtbase.h:14-22) */
     uint64_t kernel_launches;  /* kernels launched by the last render          */

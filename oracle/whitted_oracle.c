@@ -245,11 +245,13 @@ static void trace_ray(const rt_scene* s, const rt_params* p, v3 o, v3 d, int dep
             for (int k = 0; k < 3; k++) att[k] = l->color[k];
         }
         double ndl = dot4(N, L);
-        double di = ndl > 0.0 ? ndl : 0.0;           /* std::max(x, 0.0) */
+        /* std::max(x, 0.0) is (x < 0.0) ? 0.0 : x, which keeps x = -0.0: pow(-0.0, y) differs from pow(+0.0, y)
+         * for a negative odd whole y (-inf against +inf), and -V.R is -0.0 wherever V.R is exactly zero */
+        double di = ndl < 0.0 ? 0.0 : ndl;
         for (int k = 0; k < 3; k++) col[k] += di * att[k] * m->kd[k];
         v3 R = vsub(vscale(2 * dot4(N, L), N), L);
         double mvr = -dot4(d, R);
-        double si = pow(mvr > 0.0 ? mvr : 0.0, m->sp);
+        double si = pow(mvr < 0.0 ? 0.0 : mvr, m->sp);
         for (int k = 0; k < 3; k++) col[k] += si * att[k] * m->ks[k];
     }
     double kr[3] = {m->kr[0], m->kr[1], m->kr[2]};

@@ -70,6 +70,23 @@ def test_reference_shim_loop_equals_stock_renderScene(reference):
     assert np.array_equal(a, b)
 
 
+def test_oracle_keeps_a_negative_zero_like_std_max(pkg, oracle, live_reference, tmp_path):
+    """std::max(x, 0.0) is (x < 0.0) ? 0.0 : x, so it hands x = -0.0 on, and pow(-0.0, -1) is -inf.  On the centre
+    column of test_gpu_shading's axis-aligned wall -V.R is exactly -0.0: with sp = -1 the reference's specular term
+    is -inf there, with sp = -2 it is +inf.  Without the live reference this pins the oracle to the semantics of
+    std::max as the C++ standard defines it; where the reference is built, the frame must also equal its own."""
+    from test_gpu_shading import H_AX, W_AX, exponent_scene, write_scene
+    for sp, inf in ((-1.0, -np.inf), (-2.0, np.inf)):
+        sc, path = write_scene(pkg, tmp_path, f"sp_{sp}.rti", exponent_scene(sp))
+        rgb, _, _, _ = oracle.render(sc.flat, W_AX, H_AX, 2, ids=False)
+        centre = rgb[:, W_AX // 2, 0]
+        assert (centre == inf).any() and not (centre == -inf).any()
+        if live_reference is not None:
+            r_rgb, _, _, _ = live_reference.render(live_reference.load(path), W_AX, H_AX, 2, threads=2)
+            assert np.array_equal(rgb, r_rgb, equal_nan=True)
+            assert np.array_equal(np.signbit(rgb), np.signbit(r_rgb))
+
+
 GOLDEN_FULL = {"01": 1000, "05": 1000, "06": 1000, "07": 1000, "08": 1000, "09": 2000}
 
 
